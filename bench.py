@@ -2,13 +2,15 @@
 """Benchmark of the GCN-layer hot path (BASELINE.json metric: GCN layer fwd+bwd edges/sec).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload products|reddit|cbg|papers]
+                    [--dump-outputs DIR]
 
 Default workload = BASELINE.json configs[3], the largest single-GPU configuration: the ogbn-products-shaped R-MAT
 graph (N = 2 449 029, 62.8 M stored entries) under the named 3-layer model 100 -> 256 -> 256 -> 47, written as the
 reference writes its 3-layer GCN (`x = F.relu(self.gcK(x, adj))` three times, pygcn/models.py:102-111).
 One "step" = forward + backward of every layer of the workload's model (pygcn/layers.py:32-38 + autograd) over the
 whole graph; `value` = layers x stored entries / step time (layer fwd+bwd edges per second).
-Prints ONE JSON line (rank 0).  See DESIGN.md "Measurement".
+Prints ONE JSON line (rank 0).  See DESIGN.md "Measurement".  The inputs (edges, X, G, parameters) are drawn from fixed
+seeds, so two builds run with the same arguments can be compared on the files --dump-outputs writes.
 """
 from __future__ import annotations
 
@@ -47,6 +49,7 @@ WORKLOADS = {
 for _w in WORKLOADS.values():  # (tools/ read the first layer's widths)
     _w["fin"], _w["fout"] = _w["dims"][0], _w["dims"][1]
 L2_FLUSH_BYTES = 512 << 20  # > 126 MB L2
+DUMP_OUT_BYTES = 48 << 20  # --dump-outputs: the output's share; with the gradients the files stay under 64 MiB
 METRIC = "gcn_layer_fwd_bwd_edges_per_sec"
 
 
@@ -369,8 +372,9 @@ def stack_step(layers, x, graph, g):
     return h
 
 
-def capture(torch, fn):
-    """fn() captured in a CUDA graph after two eager runs on a side stream; None if capture fails."""
+def capture(torch, fn, keep=None):
+    """fn() captured in a CUDA graph after two eager runs on a side stream; None if capture fails.  keep: a dict that
+    receives under "out" the tensor the captured fn() returned (detached), which every replay rewrites."""
     try:
         s = torch.cuda.Stream()
         s.wait_stream(torch.cuda.current_stream())
@@ -381,7 +385,10 @@ def capture(torch, fn):
         torch.cuda.synchronize()
         cg = torch.cuda.CUDAGraph()
         with torch.cuda.graph(cg):
-            fn()
+            if keep is None:
+                fn()
+            else:
+                keep["out"] = fn().detach()  # (only the output's storage is held: fn's autograd graph goes as before)
         torch.cuda.synchronize()
         return cg
     except Exception as e:  # pragma: no cover
@@ -404,9 +411,30 @@ def spmm_plan(dims):
     return plan
 
 
-def measure_single(torch, P, _lib, lib, wl, dev, steps, warm, timer, full=True, use_graph=True):
+def dump_outputs(torch, outdir, out, layers):
+    """What one step returns to its caller, as float32 .npy files under outdir: `out` (the model's output; a fixed,
+    seeded sample of its rows, in row order, when the whole output exceeds DUMP_OUT_BYTES) and every layer's
+    `layer<i>_weight_grad` / `layer<i>_bias_grad`."""
+    import numpy as np
+
+    os.makedirs(outdir, exist_ok=True)
+    n, f = out.shape
+    rows = min(n, DUMP_OUT_BYTES // (4 * f))
+    if rows < n:
+        pick = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:rows].sort().values
+        out = out[pick.to(out.device)]
+    arrays = {"out": out}
+    for i, l in enumerate(layers, 1):
+        arrays["layer%d_weight_grad" % i] = l.weight.grad
+        arrays["layer%d_bias_grad" % i] = l.bias.grad
+    for name, a in arrays.items():
+        np.save(os.path.join(outdir, name + ".npy"), a.detach().float().cpu().numpy())
+
+
+def measure_single(torch, P, _lib, lib, wl, dev, steps, warm, timer, full=True, use_graph=True, dump_dir=None):
     """One workload on one GPU: graph build, the model's step (CUDA-graph replay, L2 flushed), the SpMM alone at every
-    width the step uses.  Returns (result dict, objects kept for the other sections of the line)."""
+    width the step uses.  dump_dir: write the last timed step's output and gradients there (dump_outputs).  Returns
+    (result dict, objects kept for the other sections of the line)."""
     dims, relu = wl["dims"], wl["relu"]
     n = wl["n"]
     t0 = time.perf_counter()
@@ -435,9 +463,15 @@ def measure_single(torch, P, _lib, lib, wl, dev, steps, warm, timer, full=True, 
     c0 = lib.gcnb_launch_count()
     step_eager()
     launches_per_step = int(lib.gcnb_launch_count() - c0)
-    cg = capture(torch, step_eager) if use_graph else None
-    step = cg.replay if cg is not None else step_eager
+    last = {}  # the output of the last timed step, for dump_outputs
+    cg = capture(torch, step_eager, keep=last) if use_graph else None
+
+    def step_eager_kept():
+        last["out"] = step_eager().detach()
+    step = cg.replay if cg is not None else step_eager_kept
     ms_per_step, _ = timer.time(step, steps, warm=max(warm, 3))
+    if dump_dir is not None:
+        dump_outputs(torch, dump_dir, last["out"], layers)
     res = {"ms_per_step": ms_per_step, "value": layers_n * nnz / (ms_per_step * 1e-3), "nnz": nnz, "n": n,
            "cuda_graph": cg is not None, "graph_build_s": build_s, "host_edge_generation_s": edges_s,
            "launches_per_step": launches_per_step, "bins": graph.bin_rows, "long_chunks": graph.n_long_chunks,
@@ -515,6 +549,8 @@ def run_ours(args, wl):
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     if world > 1:
+        if args.dump_outputs is not None:
+            raise SystemExit("--dump-outputs writes the outputs of a single-GPU run")
         from pygcn_b200 import dist as D
 
         return D.bench_main(args, wl)
@@ -536,7 +572,7 @@ def run_ours(args, wl):
     sampler.in_region = True  # (the clock samples that count are those taken while the step is being timed)
     wall0 = time.perf_counter()
     res, keep = measure_single(torch, P, _lib, lib, wl, dev, args.steps, warm, timer, full=True,
-                               use_graph=not args.no_cuda_graph)
+                               use_graph=not args.no_cuda_graph, dump_dir=args.dump_outputs)
     wall = time.perf_counter() - wall0
     sampler.in_region = False
     graph, layers, params = keep["graph"], keep["layers"], keep["params"]
@@ -769,9 +805,16 @@ def main():
     ap.add_argument("--no-cuda-graph", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the brief runs of the other single-GPU configs")
     ap.add_argument("--quick", action="store_true", help="N > 1: device-timed step only (no end-to-end loop, no parity gate): tuning runs")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="single GPU, --impl ours: after the timed steps, write the last step's output (a seeded "
+                         "sample of its rows when larger than 48 MiB) and every dW / db as float32 DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     wl = WORKLOADS[args.workload]
     if args.impl == "reference":
+        if args.dump_outputs is not None:
+            ap.error("--dump-outputs writes the outputs of --impl ours")
         return run_reference(args, wl)
     return run_ours(args, wl)
 
