@@ -73,10 +73,11 @@ __device__ __forceinline__ void fma_chunk(float4* acc, float v, const uint4& x) 
 
 // U gathered rows per lane in flight: all loads are issued before the first FMA (memory-level
 // parallelism is what this kernel lives on).  Entry s = (j + u) * G + slot of the current block
-// of 32; lanes past the end of the row carry v = 0 / c = 0 and are never asked for here.
+// of cnt; slots past the end of the row carry v = 0 / c = 0: their gather of row 0 is harmless,
+// their FMA is skipped (0 * Inf would put a NaN that is not in the product into the row).
 template <int LPR, int CH, int U, bool BF16>
 __device__ __forceinline__ void gather_batch(float4 (&acc)[CH * Panel<BF16>::kAcc], int c, float v, int j, int slot,
-                                             const typename Panel<BF16>::elem_t* __restrict__ b,
+                                             int cnt, const typename Panel<BF16>::elem_t* __restrict__ b,
                                              const int (&qoff)[CH], int64_t ldb) {
   constexpr int G = 32 / LPR;
   constexpr int A = Panel<BF16>::kAcc;
@@ -97,8 +98,10 @@ __device__ __forceinline__ void gather_batch(float4 (&acc)[CH * Panel<BF16>::kAc
   }
 #pragma unroll
   for (int u = 0; u < U; ++u)
+    if ((j + u) * G + slot < cnt) {
 #pragma unroll
-    for (int k = 0; k < CH; ++k) fma_vec(&acc[k * A], vv[u], x[u][k]);
+      for (int k = 0; k < CH; ++k) fma_vec(&acc[k * A], vv[u], x[u][k]);
+    }
 }
 
 // Accumulate stored entries [start, end) of one row into acc (per-lane partial sums).
@@ -135,12 +138,12 @@ __device__ __forceinline__ void accumulate_range(float4 (&acc)[CH * Panel<BF16>:
       vn = __ldg(val + base + 32 + lane);
     }
     const int cnt = min(32, end - base);
-    const int jmax = (cnt + G - 1) / G;  // entries past cnt have v = 0, c = 0: harmless
+    const int jmax = (cnt + G - 1) / G;  // entries past cnt have v = 0, c = 0 and are skipped by gather_batch
     int j = 0;
-    for (; j + U <= jmax; j += U) gather_batch<LPR, CH, U, BF16>(acc, c, v, j, slot, b, qoff, ldb);
-    if (U > 4 && j + 4 <= jmax) { gather_batch<LPR, CH, (U > 4 ? 4 : 1), BF16>(acc, c, v, j, slot, b, qoff, ldb); j += 4; }
-    if (U > 2 && j + 2 <= jmax) { gather_batch<LPR, CH, (U > 2 ? 2 : 1), BF16>(acc, c, v, j, slot, b, qoff, ldb); j += 2; }
-    if (U > 1 && j < jmax) { gather_batch<LPR, CH, 1, BF16>(acc, c, v, j, slot, b, qoff, ldb); j += 1; }
+    for (; j + U <= jmax; j += U) gather_batch<LPR, CH, U, BF16>(acc, c, v, j, slot, cnt, b, qoff, ldb);
+    if (U > 4 && j + 4 <= jmax) { gather_batch<LPR, CH, (U > 4 ? 4 : 1), BF16>(acc, c, v, j, slot, cnt, b, qoff, ldb); j += 4; }
+    if (U > 2 && j + 2 <= jmax) { gather_batch<LPR, CH, (U > 2 ? 2 : 1), BF16>(acc, c, v, j, slot, cnt, b, qoff, ldb); j += 2; }
+    if (U > 1 && j < jmax) { gather_batch<LPR, CH, 1, BF16>(acc, c, v, j, slot, cnt, b, qoff, ldb); j += 1; }
     c = cn;
     v = vn;
   }
@@ -316,7 +319,8 @@ spmm_group_kernel(int n_rows, const int32_t* __restrict__ rowptr, const uint2* _
   uint32_t nxt = cur + kBufBytes;
 
   // stage <- the next E pairs of this group's row, global -> shared; pairs past the row's end are
-  // zero-filled (col 0, val 0).  `ahead` = entries not yet staged, counted from this lane's first one.
+  // zero-filled (col 0, val 0) and gathered but not accumulated.  `ahead` = entries not yet staged, counted
+  // from this lane's first one.
   auto fetch = [&](uint32_t dst_buf, int ahead) {
 #pragma unroll
     for (int k = 0; k < NC; ++k) {
@@ -345,24 +349,21 @@ spmm_group_kernel(int n_rows, const int32_t* __restrict__ rowptr, const uint2* _
   float4 acc[A];
 #pragma unroll
   for (int t = 0; t < A; ++t) acc[t] = make_float4(0.f, 0.f, 0.f, 0.f);
-  bool first = true;
   while (!__all_sync(kFull, left <= 0)) {
     fetch(nxt, left - E - 2 * sub);  // next stage flies while this one is consumed
     cp_async_wait<1>();              // this lane's copies for the current stage have landed ...
     __syncwarp();                    // ... and so have the other lanes'
-    if (first) {  // an odd row start: the window's first pair belongs to the previous row -> value 0
-      if (lead && sub == 0) asm volatile("st.shared.u32 [%0], %1;" ::"r"(cur + 4u), "r"(0u) : "memory");
-      __syncwarp();
-      first = false;
-    }
+    // live entries of this stage: [lead, cnt) -- with an odd row start the first stage's first pair belongs to
+    // the previous row
     const int cnt = min(max(left, 0), E);
     const int cmax = __reduce_max_sync(kFull, cnt);
     // (unroll 1: with the batches unrolled ptxas software-pipelines them with 2-3 gathers in flight)
 #pragma unroll 1
     for (int j = 0; j < cmax; j += U) {
       // groups whose row has ended sit the batch out (a divergent branch, reconverged below); inside a
-      // live batch the entries past the row's end are the zero-filled pairs: at most U-1 harmless
-      // gathers of row 0 per row instead of per-gather predicates
+      // live batch the entries past the row's end (and the previous row's pair in front of an odd start)
+      // are still gathered -- at most U harmless loads per row, all of a batch in flight together -- but
+      // their FMAs are predicated off: a zero value times an Inf / NaN of the gathered row is NaN
       if (j < cnt) {
         uint4 q[U / 2];
         uint4 x[U];
@@ -383,12 +384,13 @@ spmm_group_kernel(int n_rows, const int32_t* __restrict__ rowptr, const uint2* _
         }
 #pragma unroll
         for (int h = 0; h < U / 2; ++h) {
-          fma_chunk<BF16>(acc, __uint_as_float(q[h].y), x[2 * h]);
-          fma_chunk<BF16>(acc, __uint_as_float(q[h].w), x[2 * h + 1]);
+          if (j + 2 * h >= lead && j + 2 * h < cnt) fma_chunk<BF16>(acc, __uint_as_float(q[h].y), x[2 * h]);
+          if (j + 2 * h + 1 < cnt) fma_chunk<BF16>(acc, __uint_as_float(q[h].w), x[2 * h + 1]);
         }
       }
     }
     __syncwarp();  // all lanes are done with `cur` before the next iteration's copies overwrite it
+    lead = 0;
     left -= E;
     const uint32_t t = cur;
     cur = nxt;
@@ -420,13 +422,14 @@ __device__ __forceinline__ void gather_batch_smem(float4 (&acc)[CH], const int32
   constexpr int G = 32 / LPR;
   int cc[U];
   float vv[U];
+  bool ok[U];
   float4 x[U][CH];
 #pragma unroll
   for (int u = 0; u < U; ++u) {
     const int s = s0 + u * G + slot;  // entry index inside the current block of 32
-    const bool ok = s < cnt;
-    cc[u] = ok ? cols[s] : 0;
-    vv[u] = ok ? vals[s] : 0.f;
+    ok[u] = s < cnt;
+    cc[u] = ok[u] ? cols[s] : 0;
+    vv[u] = ok[u] ? vals[s] : 0.f;
   }
 #pragma unroll
   for (int u = 0; u < U; ++u) {
@@ -436,8 +439,10 @@ __device__ __forceinline__ void gather_batch_smem(float4 (&acc)[CH], const int32
   }
 #pragma unroll
   for (int u = 0; u < U; ++u)
+    if (ok[u]) {  // (the gather of row 0 past the row's end is harmless, 0 * Inf in the sum is not)
 #pragma unroll
-    for (int k = 0; k < CH; ++k) fma4(acc[k], vv[u], x[u][k]);
+      for (int k = 0; k < CH; ++k) fma4(acc[k], vv[u], x[u][k]);
+    }
 }
 
 template <int LPR, int CH>
