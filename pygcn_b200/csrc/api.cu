@@ -87,7 +87,8 @@ int gemm_dispatch(int64_t m, int64_t n, int64_t k, const float* a, int64_t a_rs,
   }
   switch (gemm_route(m, n, k, a, a_rs, a_cs, b, b_rs, b_cs, c, ldc, precision)) {
     case 1:
-      return gemm_tc_rows_launch(m, n, k, a, a_rs, b, b_rs, b_cs, c, ldc, ws, ws_bytes, st, fb, fr, fused);
+      if (fused) *fused = true;
+      return gemm_tc_rows_launch(m, n, k, a, a_rs, b, b_rs, b_cs, c, ldc, ws, ws_bytes, st, fb, fr);
     case 2:
       return gemm_tc_tn_launch(m, n, k, a, a_cs, b, b_rs, c, ldc, ws, ws_bytes, st);
     default:
@@ -102,12 +103,14 @@ int gemm_dispatch(int64_t m, int64_t n, int64_t k, const float* a, int64_t a_rs,
     if (pr == 1) {
       const int64_t k4 = pad4(k);
       GCNB_TRY(pad_copy_launch(m, k, a, a_rs, pad, k4, st));
-      if (gemm_tc_rows_eligible(m, n, k4, pad, k4, 1, c, ldc) && rest_bytes >= gemm_tc_rows_workspace_bytes(m, n, k))
-        return gemm_tc_rows_launch(m, n, k, pad, k4, b, b_rs, b_cs, c, ldc, rest, rest_bytes, st, fb, fr, fused);
+      if (gemm_tc_rows_eligible(m, n, k4, pad, k4, 1, c, ldc) && rest_bytes >= gemm_tc_rows_workspace_bytes(m, n, k)) {
+        if (fused) *fused = true;
+        return gemm_tc_rows_launch(m, n, k, pad, k4, b, b_rs, b_cs, c, ldc, rest, rest_bytes, st, fb, fr);
+      }
     } else {
       const int64_t m4 = pad4(m);
       GCNB_TRY(pad_copy_launch(k, m, a, a_cs, pad, m4, st));  // X [k rows, m cols], row stride a_cs
-      if (gemm_tc_tn_eligible(m, n, k, pad, m4, b, b_rs, /*padded=*/true) &&
+      if (gemm_tc_tn_eligible(m, n, k, pad, m4, b, b_rs) &&
           rest_bytes >= gemm_tc_tn_workspace_bytes(m, n, k))
         return gemm_tc_tn_launch(m, n, k, pad, m4, b, b_rs, c, ldc, rest, rest_bytes, st);
     }
@@ -185,7 +188,7 @@ int graph_matmul(const gcnb_graph* g, bool transpose, const float* b, int64_t ld
     // path's truncating TMEM accumulation then shows as 3e-6 ... 1e-5 of the result (cuBLAS fp32: 3e-7 ... 9e-7,
     // profiles/r02_debug_ref_models.txt) -- inside the bar, but the reference's fresh BatchNorm amplifies it 100x.
     const bool big = (double)m * (double)fw * (double)r >= 4.0e9;
-    if (big && gemm_tc_tn_eligible(m, fw, r, x, ldx, b + f0, ldb, /*padded=*/true) && (f0 % 4 == 0)) {
+    if (big && gemm_tc_tn_eligible(m, fw, r, x, ldx, b + f0, ldb) && (f0 % 4 == 0)) {
       GCNB_TRY(gemm_tc_tn_launch(m, fw, r, x, ldx, b + f0, ldb, out + f0, ldo, ws, ws_bytes, st));
     } else {
       GCNB_TRY(gemm_fp32_launch(m, fw, r, x, 1, ldx, b + f0, ldb, 1, out + f0, ldo, ws, ws_bytes, st));

@@ -153,14 +153,13 @@ size_t gemm_fp32_workspace_bytes(int64_t m, int64_t n, int64_t k);
 bool gemm_tc_rows_eligible(int64_t m, int64_t n, int64_t k, const float* a, int64_t a_rs, int64_t a_cs,
                            const float* c, int64_t ldc);
 size_t gemm_tc_rows_workspace_bytes(int64_t m, int64_t n, int64_t k);
-// ep_bias / ep_relu: C = act(A B + bias) when the kernel that runs can fuse it (*ep_done = true); otherwise the
-// caller applies bias_act_launch afterwards
+// ep_bias / ep_relu: C = act(A B + bias), applied by the kernel's epilogue
 int gemm_tc_rows_launch(int64_t m, int64_t n, int64_t k, const float* a, int64_t lda, const float* b,
                         int64_t b_rs, int64_t b_cs, float* c, int64_t ldc, void* ws, size_t ws_bytes,
-                        cudaStream_t stream, const float* ep_bias = nullptr, int ep_relu = 0, bool* ep_done = nullptr);
+                        cudaStream_t stream, const float* ep_bias = nullptr, int ep_relu = 0);
 bool gemm_tc_rows_beats_skinny(int64_t k);
 bool gemm_tc_tn_eligible(int64_t m, int64_t n, int64_t r, const float* x, int64_t ldx, const float* y,
-                         int64_t ldy, bool padded = false);
+                         int64_t ldy);
 size_t gemm_tc_tn_workspace_bytes(int64_t m, int64_t n, int64_t r);
 int gemm_tc_tn_launch(int64_t m, int64_t n, int64_t r, const float* x, int64_t ldx, const float* y,
                       int64_t ldy, float* c, int64_t ldc, void* ws, size_t ws_bytes, cudaStream_t stream);

@@ -1,25 +1,25 @@
 // tcgen05 (5th-gen tensor core) GEMMs for the dense contractions of the GCN layer, fp32 in /
 // fp32 out with fp32-level accuracy through the 3-term TF32 split ("3xTF32"):
-//     a = a_hi + a_lo,  b = b_hi + b_lo   (hi = cvt.rna.tf32, lo = a - hi, exact)
+//     a = a_hi + a_lo,  b = b_hi + b_lo   (lo = a - hi, exact)
 //     a*b ~= a_lo*b_hi + a_hi*b_lo + a_hi*b_hi          (fp32 accumulate in TMEM)
 //
 //   mode R ("rows"):  C[M,N] = A[M,K] * B[K,N], A row-major with K contiguous, M huge, K/N small
 //                     support = X W (pygcn/layers.py:33) and dX = dS W^T (MmBackward0).
-//                     B is tiny: a pre-pass packs it once into hi/lo images that already have the
-//                     UMMA shared-memory layout, the main kernel pulls them with cp.async.bulk
-//                     (TMA, mbarrier complete_tx); A streams HBM -> registers -> split -> smem.
+//                     B is tiny: a pre-pass packs it once into hi/lo images (hi = cvt.rna.tf32) that
+//                     already have the UMMA shared-memory layout, the main kernel pulls them with
+//                     cp.async.bulk (TMA, mbarrier complete_tx); A arrives in K-major tiles by TMA
+//                     tensor-map loads and is split in shared memory (hi = the raw words, truncated).
 //   mode T ("tn"):    C[M,N] = sum_r X[r,M]^T * Y[r,N]: both operands row-major with the
 //                     reduction index outermost (dW = X^T dS).  Rows are split across CTAs
-//                     (split-K); tiles are transposed into K-major smem on the fly; partial
-//                     tiles are reduced in a fixed order (deterministic).
+//                     (split-K); both operands arrive by TMA as MN-major tiles and are split
+//                     the same way; partial tiles are reduced in a fixed order (deterministic).
 //
-// Every operand tile in shared memory is the canonical K-major SWIZZLE_128B layout
-// (rows of 32 tf32 = 128 B, 16-byte chunk c of row r stored at chunk c ^ (r & 7), 8-row groups
-// 1024 B apart), accumulators live in TMEM (128 lanes x N columns fp32), tcgen05.mma is issued
-// by one thread, completion is tracked with tcgen05.commit -> mbarrier, the epilogue reads TMEM
-// with tcgen05.ld.  Two smem stages; 2 CTAs per SM give the inter-tile overlap.
+// K-major operand tiles in shared memory have the canonical SWIZZLE_128B layout (rows of 32 tf32 = 128 B,
+// 16-byte chunk c of row r stored at chunk c ^ (r & 7), 8-row groups 1024 B apart), accumulators live in
+// TMEM (128 lanes x N columns fp32), tcgen05.mma is issued by one thread, completion is tracked with
+// tcgen05.commit -> mbarrier, the epilogue reads TMEM with tcgen05.ld.  Both kernels are warp-specialised
+// (TMA producer, splitters, MMA issuer, epilogue), one CTA per SM, with as many operand stages as fit.
 #include <cuda.h>  // CUtensorMap types only: the encoder is fetched with cudaGetDriverEntryPoint (no libcuda link)
-#include <stdlib.h>
 #include <string.h>
 
 #include "common.cuh"
@@ -28,8 +28,7 @@
 namespace gcnb {
 namespace {
 
-constexpr int kThreads = 256;
-constexpr int BM = 128;        // UMMA M
+constexpr int BM = 128;       // UMMA M
 constexpr int BKF = 32;        // floats per K block (one 128-byte swizzle row)
 constexpr int kTileBytes = BM * 128;  // one 128-row operand tile (hi or lo)
 constexpr int kChunkBlocks = 8;  // K blocks (of 32) accumulated inside TMEM before a drain
@@ -62,16 +61,6 @@ __device__ __forceinline__ void umma_tf32(uint32_t tmem_d, uint64_t adesc, uint6
 __device__ __forceinline__ void umma_commit(uint32_t bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
 }
-__device__ __forceinline__ void tmem_ld8(uint32_t taddr, float (&v)[8]) {
-  uint32_t r0, r1, r2, r3, r4, r5, r6, r7;
-  asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
-               : "=r"(r0), "=r"(r1), "=r"(r2), "=r"(r3), "=r"(r4), "=r"(r5), "=r"(r6), "=r"(r7)
-               : "r"(taddr));
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-  v[0] = __uint_as_float(r0); v[1] = __uint_as_float(r1); v[2] = __uint_as_float(r2); v[3] = __uint_as_float(r3);
-  v[4] = __uint_as_float(r4); v[5] = __uint_as_float(r5); v[6] = __uint_as_float(r6); v[7] = __uint_as_float(r7);
-}
-
 // K-major SWIZZLE_128B shared-memory matrix descriptor (cute::UMMA::SmemDescriptor):
 // start>>4 [0,14) | LBO>>4 [16,30) (=1, unused) | SBO>>4 [32,46) (=1024 B) | version=1 [46,48) | layout=2 [61,64)
 __device__ __forceinline__ uint64_t make_desc(uint32_t smem_addr) {
@@ -115,26 +104,6 @@ __device__ __forceinline__ uint32_t sw128_off(int r, int k) {
   return (uint32_t)(r * 128 + ((((k >> 2) ^ (r & 7)) << 4) | ((k & 3) << 2)));
 }
 
-struct Smem {
-  // offsets (bytes) into the 1024-aligned dynamic shared memory block
-  uint32_t a_hi[2], a_lo[2], b_hi[2], b_lo[2];
-  uint32_t bars;  // mma_done[2], b_full[2], accum_full  (5 x 8 bytes) then tmem slot
-};
-
-// b_slots: number of (hi, lo) B tile pairs kept in shared memory: 2 when B is streamed per K block,
-// nkb when the whole packed B fits and stays resident (slot kb at b_hi[0] + kb * 2 * npad * 128).
-__host__ __device__ inline uint32_t smem_layout(int npad, Smem* s, int b_slots = 2) {
-  uint32_t off = 0;
-  const uint32_t bt = (uint32_t)npad * 128;
-  for (int i = 0; i < 2; ++i) { s->a_hi[i] = off; off += kTileBytes; s->a_lo[i] = off; off += kTileBytes; }
-  for (int i = 0; i < 2; ++i) { s->b_hi[i] = off + (uint32_t)i * 2 * bt; s->b_lo[i] = s->b_hi[i] + bt; }
-  off += (uint32_t)b_slots * 2 * bt;
-  off = (off + 1023) & ~1023u;
-  s->bars = off;
-  off += 64;
-  return off;
-}
-
 // One K block: 4 K-steps of 8 tf32, 3 MMAs each.  first = first K block of the tile.
 __device__ __forceinline__ void issue_kblock(uint32_t tmem_d, uint32_t a_hi, uint32_t a_lo, uint32_t b_hi,
                                              uint32_t b_lo, uint32_t idesc, bool first) {
@@ -145,56 +114,6 @@ __device__ __forceinline__ void issue_kblock(uint32_t tmem_d, uint32_t a_hi, uin
     umma_tf32(tmem_d, dal + adv, dbh + adv, idesc, (first && ks == 0) ? 0u : 1u);
     umma_tf32(tmem_d, dah + adv, dbl + adv, idesc, 1u);
     umma_tf32(tmem_d, dah + adv, dbh + adv, idesc, 1u);
-  }
-}
-
-// MN-major variant: a_* tiles are 4 M-groups x 8 K-groups of 512-byte atoms (atom (mm,kg) at
-// (mm + 4*kg) * 512), b_* tiles are ng N-groups x 8 K-groups (atom (nn,kg) at (nn + ng*kg) * 512);
-// one UMMA K step (8 tf32) spans two K groups.
-__device__ __forceinline__ void issue_kblock_mn(uint32_t tmem_d, uint32_t a_hi, uint32_t a_lo, uint32_t b_hi,
-                                                uint32_t b_lo, uint32_t idesc, int ng, bool first) {
-#pragma unroll
-  for (int ks = 0; ks < BKF / 8; ++ks) {
-    const uint32_t ao = (uint32_t)ks * 4096u, bo = (uint32_t)(ks * ng) * 1024u;
-    const uint64_t dah = make_desc_mn(a_hi + ao, 512u, 2048u), dal = make_desc_mn(a_lo + ao, 512u, 2048u);
-    const uint64_t dbh = make_desc_mn(b_hi + bo, 512u, (uint32_t)ng * 512u);
-    const uint64_t dbl = make_desc_mn(b_lo + bo, 512u, (uint32_t)ng * 512u);
-    umma_tf32(tmem_d, dal, dbh, idesc, (first && ks == 0) ? 0u : 1u);
-    umma_tf32(tmem_d, dah, dbl, idesc, 1u);
-    umma_tf32(tmem_d, dah, dbh, idesc, 1u);
-  }
-}
-
-// Epilogue: TMEM accumulator (128 lanes x npad columns) -> global rows.  Warp w owns lane quarter
-// w & 3 and column half w >> 2.
-__device__ __forceinline__ void epilogue_store(uint32_t tmem_d, int npad, float* __restrict__ c, int64_t ldc,
-                                               int64_t row0, int64_t m_rows, int n0, int n_cols, bool vec_ok,
-                                               bool add = false) {
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int q = warp & 3, h = warp >> 2;
-  const int64_t row = row0 + q * 32 + lane;
-  const int half = npad >> 1;
-  for (int cb = h * half; cb < (h + 1) * half; cb += 8) {
-    float v[8];
-    __syncwarp();  // tcgen05.ld is .sync.aligned: the spin-wait above may have split the warp
-    tmem_ld8(tmem_d + ((uint32_t)(q * 32) << 16) + (uint32_t)cb, v);  // warp-collective
-    if (row < m_rows) {
-      float* dst = c + row * ldc + n0 + cb;
-      if (vec_ok && cb + 8 <= n_cols) {
-        if (add) {  // later K chunk of the same tile: fp32 round-to-nearest add outside the tensor core
-          const float4 p0 = *reinterpret_cast<const float4*>(dst);
-          const float4 p1 = *reinterpret_cast<const float4*>(dst + 4);
-          v[0] += p0.x; v[1] += p0.y; v[2] += p0.z; v[3] += p0.w;
-          v[4] += p1.x; v[5] += p1.y; v[6] += p1.z; v[7] += p1.w;
-        }
-        *reinterpret_cast<float4*>(dst) = make_float4(v[0], v[1], v[2], v[3]);
-        *reinterpret_cast<float4*>(dst + 4) = make_float4(v[4], v[5], v[6], v[7]);
-      } else {
-#pragma unroll
-        for (int t = 0; t < 8; ++t)
-          if (cb + t < n_cols) dst[t] = add ? dst[t] + v[t] : v[t];
-      }
-    }
   }
 }
 
@@ -229,324 +148,10 @@ pack_b_kernel(int64_t K, int64_t N, int npad, int n_tiles, int nkb, const float*
 }
 
 // ------------------------------------------------------------------ mode R kernel
-__global__ void __launch_bounds__(kThreads, 2)
-gemm_tc_rows_kernel(int64_t M, int N, int K, const float* __restrict__ a, int64_t lda,
-                    const float* __restrict__ img_hi, const float* __restrict__ img_lo, float* __restrict__ c,
-                    int64_t ldc, int npad, int nkb, int tmem_cols, int vec_ok, int b_resident) {
-  extern __shared__ __align__(1024) uint8_t smem_raw[];
-  const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
-  Smem L;
-  smem_layout(npad, &L, b_resident ? nkb : 2);
-  const uint32_t bar_mma[2] = {base + L.bars, base + L.bars + 8};
-  const uint32_t bar_b[2] = {base + L.bars + 16, base + L.bars + 24};
-  const uint32_t bar_acc = base + L.bars + 32;
-  const uint32_t tmem_slot = base + L.bars + 40;
-  uint8_t* gen = smem_raw + (base - smem_u32(smem_raw));  // generic pointer to the aligned block
-
-  const int tid = threadIdx.x;
-  if (tid == 0) {
-    mbar_init(bar_mma[0], 1); mbar_init(bar_mma[1], 1);
-    mbar_init(bar_b[0], 1); mbar_init(bar_b[1], 1);
-    mbar_init(bar_acc, 1);
-    fence_barrier_init();
-  }
-  if (tid < 32) {
-    __syncwarp();
-    tmem_alloc(tmem_slot, (uint32_t)tmem_cols);
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_d = *reinterpret_cast<volatile uint32_t*>(gen + L.bars + 40);
-  const uint32_t idesc = make_idesc(npad);
-  const uint32_t b_bytes = (uint32_t)npad * 128;
-
-  const int nt = blockIdx.y;           // N tile (npad columns)
-  if (b_resident && tid == 0) {
-    // the whole packed B (hi and lo images of every K block) is pulled once with TMA bulk copies
-    // and stays in shared memory: no per-K-block fetch on the MMA critical path
-    mbar_expect_tx(bar_b[0], 2 * b_bytes * (uint32_t)nkb);
-    for (int kb = 0; kb < nkb; ++kb) {
-      const int64_t blk = (int64_t)nt * nkb + kb;
-      bulk_g2s(base + L.b_hi[0] + (uint32_t)kb * 2 * b_bytes, img_hi + blk * ((int64_t)npad * BKF), b_bytes, bar_b[0]);
-      bulk_g2s(base + L.b_lo[0] + (uint32_t)kb * 2 * b_bytes, img_lo + blk * ((int64_t)npad * BKF), b_bytes, bar_b[0]);
-    }
-  }
-  bool b_ready = false;
-  const int n0 = nt * npad;
-  const int n_cols = min(npad, N - n0);
-  const int64_t m_tiles = (M + BM - 1) / BM;
-
-  // thread -> (row, 16-byte chunk) of the A tile: 8 threads cover one 128-byte row segment
-  const int chunk = tid & 7;
-  const int row_in = tid >> 3;  // 0..31, +32*j
-  uint32_t it = 0;              // K-block iteration counter across tiles (stage = it & 1)
-  uint32_t acc_parity = 0;
-
-  // A tile loads run two K blocks ahead of the split (cur <- n1 <- n2) over the flattened
-  // (tile, K block) sequence of this CTA, so the prefetch crosses tile boundaries and the epilogue
-  // of a tile overlaps the next tile's loads: ~3 x 16 KB in flight per CTA, 2 CTAs per SM.
-  const int64_t my_tiles = (m_tiles > (int64_t)blockIdx.x) ? (m_tiles - blockIdx.x + gridDim.x - 1) / gridDim.x : 0;
-  const int64_t n_items = my_tiles * nkb;
-  auto load_item = [&](int64_t item, float4 (&dst)[4]) {
-    const int64_t m0 = ((int64_t)blockIdx.x + (item / nkb) * gridDim.x) * BM;
-    const int kb = (int)(item % nkb);
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-      const int64_t r = m0 + row_in + 32 * j;
-      const int k = kb * BKF + chunk * 4;
-      dst[j] = make_float4(0.f, 0.f, 0.f, 0.f);
-      if (r < M && k < K) dst[j] = __ldg(reinterpret_cast<const float4*>(a + r * lda + k));
-    }
-  };
-  float4 cur[4], n1[4], n2[4];
-  if (n_items > 0) load_item(0, cur);
-  if (n_items > 1) load_item(1, n1);
-  int64_t item = 0;
-  for (int64_t mt = blockIdx.x; mt < m_tiles; mt += gridDim.x) {
-    const int64_t m0 = mt * BM;
-    for (int kb = 0; kb < nkb; ++kb, ++it, ++item) {
-      const int s = it & 1;
-      const uint32_t use = it >> 1;  // n-th use of stage s
-      if (item + 2 < n_items) load_item(item + 2, n2);
-      if (use > 0) mbar_wait(bar_mma[s], (use - 1) & 1);  // MMAs that read stage s have retired
-      if (tid == 0 && !b_resident) {
-        mbar_expect_tx(bar_b[s], 2 * b_bytes);
-        const int64_t blk = (int64_t)nt * nkb + kb;
-        bulk_g2s(base + L.b_hi[s], img_hi + blk * ((int64_t)npad * BKF), b_bytes, bar_b[s]);
-        bulk_g2s(base + L.b_lo[s], img_lo + blk * ((int64_t)npad * BKF), b_bytes, bar_b[s]);
-      }
-#pragma unroll
-      for (int j = 0; j < 4; ++j) {
-        const int r = row_in + 32 * j;
-        float4 hi, lo;
-        split_tf32(cur[j].x, hi.x, lo.x); split_tf32(cur[j].y, hi.y, lo.y);
-        split_tf32(cur[j].z, hi.z, lo.z); split_tf32(cur[j].w, hi.w, lo.w);
-        const uint32_t off = (uint32_t)(r * 128 + ((chunk ^ (r & 7)) << 4));
-        *reinterpret_cast<float4*>(gen + L.a_hi[s] + off) = hi;
-        *reinterpret_cast<float4*>(gen + L.a_lo[s] + off) = lo;
-      }
-      fence_proxy_async();
-      __syncthreads();
-      if (tid == 0) {
-        uint32_t bh = base + L.b_hi[s], bl = base + L.b_lo[s];
-        if (b_resident) {
-          if (!b_ready) { mbar_wait(bar_b[0], 0); b_ready = true; }
-          bh = base + L.b_hi[0] + (uint32_t)kb * 2 * b_bytes;
-          bl = base + L.b_lo[0] + (uint32_t)kb * 2 * b_bytes;
-        } else {
-          mbar_wait(bar_b[s], use & 1);
-        }
-        tc_fence_after();
-        issue_kblock(tmem_d, base + L.a_hi[s], base + L.a_lo[s], bh, bl, idesc,
-                     kb % kChunkBlocks == 0);
-        umma_commit(bar_mma[s]);
-        if (kb == nkb - 1 || kb % kChunkBlocks == kChunkBlocks - 1) umma_commit(bar_acc);
-      }
-#pragma unroll
-      for (int j = 0; j < 4; ++j) {
-        cur[j] = n1[j];
-        n1[j] = n2[j];
-      }
-      if (kb == nkb - 1 || kb % kChunkBlocks == kChunkBlocks - 1) {
-        // drain the accumulator every kChunkBlocks K blocks: the tensor core adds into TMEM with
-        // truncation, so long reductions are finished with fp32 RN adds in the epilogue instead
-        mbar_wait(bar_acc, acc_parity);
-        acc_parity ^= 1;
-        tc_fence_after();
-        epilogue_store(tmem_d, npad, c, ldc, m0, M, n0, n_cols, vec_ok != 0, kb >= kChunkBlocks);
-        tc_fence_before();
-        __syncthreads();
-      }
-    }
-  }
-  if (tid < 32) {
-    __syncwarp();
-    tmem_dealloc(tmem_d, (uint32_t)tmem_cols);
-  }
-}
-
-// ------------------------------------------------------------------ mode R kernel, warp specialised
-// Same product and data path as gemm_tc_rows_kernel, restructured as the canonical Blackwell
-// pipeline: the three stages only meet through mbarriers, so loads, tensor-core work and the
-// TMEM drain of different tiles overlap inside one CTA (one CTA per SM, persistent over M tiles).
-//   warps 0-3  epilogue   : wait acc_full[a] -> tcgen05.ld lanes 32w..32w+31 -> global -> arrive acc_empty[a]
-//   warp  4    MMA issuer : TMEM alloc; resident B via TMA; wait full[s] -> 12 x tcgen05.mma ->
-//                           tcgen05.commit -> empty[s]; per K chunk commit -> acc_full[a]
-//   warps 5-8  producers  : HBM -> registers (one item ahead) -> (hi, lo) -> SW128 smem stage s ->
-//                           fence.proxy.async -> arrive full[s]
-// NS operand stages of 32 KB, two TMEM accumulators of npad columns.  Requires resident B.
-constexpr int kWsThreads = 288;
-
-__global__ void __launch_bounds__(kWsThreads, 1)
-gemm_tc_rows_ws_kernel(int64_t M, int N, int K, const float* __restrict__ a, int64_t lda,
-                       const float* __restrict__ img_hi, const float* __restrict__ img_lo, float* __restrict__ c,
-                       int64_t ldc, int npad, int nkb, int tmem_cols, int vec_ok, int ns) {
-  extern __shared__ __align__(1024) uint8_t smem_raw[];
-  const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
-  uint8_t* gen = smem_raw + (base - smem_u32(smem_raw));
-  // layout: [ns x (a_hi 16K, a_lo 16K)] [nkb x (b_hi, b_lo)] [barriers]
-  const uint32_t b_bytes = (uint32_t)npad * 128;
-  const uint32_t off_b = (uint32_t)ns * 2 * kTileBytes;
-  const uint32_t off_bar = (off_b + (uint32_t)nkb * 2 * b_bytes + 1023u) & ~1023u;
-  auto bar_full = [&](int s_) { return base + off_bar + 8u * (uint32_t)s_; };
-  auto bar_empty = [&](int s_) { return base + off_bar + 64u + 8u * (uint32_t)s_; };
-  const uint32_t bar_b = base + off_bar + 128u;
-  auto bar_acc_full = [&](int a_) { return base + off_bar + 136u + 8u * (uint32_t)a_; };
-  auto bar_acc_empty = [&](int a_) { return base + off_bar + 152u + 8u * (uint32_t)a_; };
-  const uint32_t tmem_slot_off = off_bar + 168u;
-
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  if (tid == 0) {
-    for (int i = 0; i < ns; ++i) { mbar_init(bar_full(i), 4); mbar_init(bar_empty(i), 1); }
-    mbar_init(bar_b, 1);
-    for (int i = 0; i < 2; ++i) { mbar_init(bar_acc_full(i), 1); mbar_init(bar_acc_empty(i), 4); }
-    fence_barrier_init();
-  }
-  if (warp == 4) {
-    __syncwarp();
-    tmem_alloc(base + tmem_slot_off, (uint32_t)tmem_cols);
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *reinterpret_cast<volatile uint32_t*>(gen + tmem_slot_off);
-
-  const int nt = blockIdx.y;
-  const int n0 = nt * npad;
-  const int n_cols = min(npad, N - n0);
-  const int64_t m_tiles = (M + BM - 1) / BM;
-  const int64_t my_tiles = (m_tiles > (int64_t)blockIdx.x) ? (m_tiles - blockIdx.x + gridDim.x - 1) / gridDim.x : 0;
-  const int64_t n_items = my_tiles * nkb;
-  const int chunks_per_tile = (nkb + kChunkBlocks - 1) / kChunkBlocks;
-
-  if (warp >= 5) {
-    // ===================== producers =====================
-    const int pt = tid - 160;
-    const int chunk = pt & 7;
-    const int row_in = pt >> 3;  // 0..15, +16*j
-    auto load_item = [&](int64_t item, float4 (&dst)[8]) {
-      const int64_t m0 = ((int64_t)blockIdx.x + (item / nkb) * gridDim.x) * BM;
-      const int k = (int)(item % nkb) * BKF + chunk * 4;
-#pragma unroll
-      for (int j = 0; j < 8; ++j) {
-        const int64_t r = m0 + row_in + 16 * j;
-        dst[j] = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (r < M && k < K) dst[j] = __ldg(reinterpret_cast<const float4*>(a + r * lda + k));
-      }
-    };
-    float4 cur[8], nxt[8];
-    if (n_items > 0) load_item(0, cur);
-    for (int64_t item = 0; item < n_items; ++item) {
-      const int s = (int)(item % ns);
-      const uint32_t use = (uint32_t)(item / ns);
-      if (item + 1 < n_items) load_item(item + 1, nxt);
-      if (use > 0) mbar_wait(bar_empty(s), (use - 1) & 1);
-      uint8_t* a_hi = gen + (uint32_t)s * 2 * kTileBytes;
-      uint8_t* a_lo = a_hi + kTileBytes;
-#pragma unroll
-      for (int j = 0; j < 8; ++j) {
-        const int r = row_in + 16 * j;
-        float4 hi, lo;
-        split_tf32(cur[j].x, hi.x, lo.x); split_tf32(cur[j].y, hi.y, lo.y);
-        split_tf32(cur[j].z, hi.z, lo.z); split_tf32(cur[j].w, hi.w, lo.w);
-        const uint32_t off = (uint32_t)(r * 128 + ((chunk ^ (r & 7)) << 4));
-        *reinterpret_cast<float4*>(a_hi + off) = hi;
-        *reinterpret_cast<float4*>(a_lo + off) = lo;
-      }
-      fence_proxy_async();
-      __syncwarp();
-      if (lane == 0) mbar_arrive(bar_full(s));
-#pragma unroll
-      for (int j = 0; j < 8; ++j) cur[j] = nxt[j];
-    }
-  } else if (warp == 4) {
-    // ===================== MMA issuer =====================
-    if (lane == 0) {
-      const uint32_t idesc = make_idesc(npad);
-      mbar_expect_tx(bar_b, 2 * b_bytes * (uint32_t)nkb);
-      for (int kb = 0; kb < nkb; ++kb) {
-        const int64_t blk = (int64_t)nt * nkb + kb;
-        bulk_g2s(base + off_b + (uint32_t)kb * 2 * b_bytes, img_hi + blk * ((int64_t)npad * BKF), b_bytes, bar_b);
-        bulk_g2s(base + off_b + (uint32_t)kb * 2 * b_bytes + b_bytes, img_lo + blk * ((int64_t)npad * BKF), b_bytes,
-                 bar_b);
-      }
-      mbar_wait(bar_b, 0);
-      int64_t item = 0;
-      uint32_t chunk_ctr = 0;
-      for (int64_t t = 0; t < my_tiles; ++t) {
-        for (int kb = 0; kb < nkb; ++kb, ++item) {
-          const int ab = (int)(chunk_ctr & 1u);
-          const uint32_t j_use = chunk_ctr >> 1;
-          if (kb % kChunkBlocks == 0 && j_use > 0) mbar_wait(bar_acc_empty(ab), (j_use - 1) & 1);
-          const int s = (int)(item % ns);
-          const uint32_t use = (uint32_t)(item / ns);
-          mbar_wait(bar_full(s), use & 1);
-          tc_fence_after();
-          const uint32_t a_hi = base + (uint32_t)s * 2 * kTileBytes;
-          const uint32_t bh = base + off_b + (uint32_t)kb * 2 * b_bytes;
-          issue_kblock(tmem_base + (uint32_t)ab * (uint32_t)npad, a_hi, a_hi + kTileBytes, bh, bh + b_bytes, idesc,
-                       kb % kChunkBlocks == 0);
-          umma_commit(bar_empty(s));
-          if (kb == nkb - 1 || kb % kChunkBlocks == kChunkBlocks - 1) {
-            umma_commit(bar_acc_full(ab));
-            ++chunk_ctr;
-          }
-        }
-      }
-    }
-  } else {
-    // ===================== epilogue =====================
-    uint32_t chunk_ctr = 0;
-    for (int64_t t = 0; t < my_tiles; ++t) {
-      const int64_t m0 = ((int64_t)blockIdx.x + t * gridDim.x) * BM;
-      const int64_t row = m0 + warp * 32 + lane;
-      for (int ch = 0; ch < chunks_per_tile; ++ch, ++chunk_ctr) {
-        const int ab = (int)(chunk_ctr & 1u);
-        mbar_wait(bar_acc_full(ab), (chunk_ctr >> 1) & 1);
-        tc_fence_after();
-        const bool add = ch > 0;
-        for (int cb = 0; cb < npad; cb += 8) {
-          float v[8];
-          __syncwarp();
-          tmem_ld8(tmem_base + (uint32_t)ab * (uint32_t)npad + ((uint32_t)(warp * 32) << 16) + (uint32_t)cb, v);
-          if (row < M) {
-            float* dst = c + row * ldc + n0 + cb;
-            if (vec_ok && cb + 8 <= n_cols) {
-              if (add) {
-                const float4 p0 = *reinterpret_cast<const float4*>(dst);
-                const float4 p1 = *reinterpret_cast<const float4*>(dst + 4);
-                v[0] += p0.x; v[1] += p0.y; v[2] += p0.z; v[3] += p0.w;
-                v[4] += p1.x; v[5] += p1.y; v[6] += p1.z; v[7] += p1.w;
-              }
-              *reinterpret_cast<float4*>(dst) = make_float4(v[0], v[1], v[2], v[3]);
-              *reinterpret_cast<float4*>(dst + 4) = make_float4(v[4], v[5], v[6], v[7]);
-            } else {
-#pragma unroll
-              for (int t2 = 0; t2 < 8; ++t2)
-                if (cb + t2 < n_cols) dst[t2] = add ? dst[t2] + v[t2] : v[t2];
-            }
-          }
-        }
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive(bar_acc_empty(ab));
-      }
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 4) {
-    __syncwarp();
-    tmem_dealloc(tmem_base, (uint32_t)tmem_cols);
-  }
-}
-
-// ------------------------------------------------------------------ mode R kernel, TMA-fed
-// The two kernels above move A through registers: HBM -> LDG -> split -> STS.  A thread can keep only one or
-// two 16 KB K blocks ahead that way (16-48 KB in flight per SM), and measured 1.7 TB/s on the shapes that
-// are pure streams (papers100M-shaped 13.8 M x 128 -> 128: 8.2 ms for 14.1 GB).  Here the copy engine does
-// the streaming and the SM only does arithmetic:
+// A moved through registers (HBM -> LDG -> split -> STS) keeps only one or two 16 KB K blocks ahead per thread
+// (16-48 KB in flight per SM): such a kernel measured 1.7 TB/s on the shapes that are pure streams
+// (papers100M-shaped 13.8 M x 128 -> 128: 8.2 ms for 14.1 GB).  Here the copy engine does the streaming and the
+// SM only does arithmetic:
 //   warp  5    TMA producer: one thread issues cp.async.bulk.tensor.2d per (M tile, K block): a 128 x 32 fp32
 //              box of A, SWIZZLE_128B, lands in stage s as the K-major UMMA tile; rows / columns past the
 //              matrix are zero-filled by the tensor map.  With ns stages, (ns-1) x 16 KB stay in flight.
@@ -554,12 +159,12 @@ gemm_tc_rows_ws_kernel(int64_t M, int N, int K, const float* __restrict__ a, int
 //   warps 6-9  splitters: wait raw_full[s]; a_lo = a - tf32(a) written to the stage's second tile at the SAME
 //              byte offsets (the swizzle is a property of the address, so no index arithmetic); the raw tile
 //              itself is the hi operand -- kind::tf32 reads the upper 19 bits of each word, i.e. truncates, and
-//              a - trunc(a) is exact in fp32 (hi_rna = 1 instead overwrites the raw tile with cvt.rna values).
+//              a - trunc(a) is exact in fp32.
 //   warp  4    MMA issuer (one thread): 12 tcgen05.mma per K block into one of two TMEM accumulators,
 //              tcgen05.commit -> empty[s] / acc_full[a].
 //   warps 0-3  epilogue: tcgen05.ld 32 columns -> registers -> per-warp shared staging (row stride 36 floats,
 //              conflict free) -> global stores in which 8 lanes write one full 128-byte line of a C row
-//              (the lane-per-row stores of the kernels above touch 32 lines per instruction).
+//              (lane-per-row stores would touch 32 lines per instruction).
 constexpr int kTmaThreads = 320;
 constexpr int kEpiLd = 36;
 constexpr int kTmaMaxStages = 8;
@@ -588,7 +193,7 @@ template <bool PDL>
 __global__ void __launch_bounds__(kTmaThreads, 1)
 gemm_tc_rows_tma_kernel(const __grid_constant__ TmaDesc tmap_a, int64_t M, int N, int K,
                         const float* __restrict__ img_hi, const float* __restrict__ img_lo, float* __restrict__ c,
-                        int64_t ldc, int npad, int nkb, int tmem_cols, int vec_ok, int ns, int b_resident, int hi_rna,
+                        int64_t ldc, int npad, int nkb, int tmem_cols, int vec_ok, int ns, int b_resident,
                         const float* __restrict__ ep_bias, int ep_relu) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
@@ -678,17 +283,11 @@ gemm_tc_rows_tma_kernel(const __grid_constant__ TmaDesc tmap_a, int64_t M, int N
       for (int j = 0; j < 8; ++j) {
         const uint32_t off = 16u * (uint32_t)(pt + 128 * j);
         const float4 v = *reinterpret_cast<const float4*>(raw + off);
-        float4 hi, lo;
-        if (hi_rna) {
-          split_tf32(v.x, hi.x, lo.x); split_tf32(v.y, hi.y, lo.y);
-          split_tf32(v.z, hi.z, lo.z); split_tf32(v.w, hi.w, lo.w);
-          *reinterpret_cast<float4*>(raw + off) = hi;
-        } else {
-          lo.x = v.x - __uint_as_float(__float_as_uint(v.x) & 0xffffe000u);
-          lo.y = v.y - __uint_as_float(__float_as_uint(v.y) & 0xffffe000u);
-          lo.z = v.z - __uint_as_float(__float_as_uint(v.z) & 0xffffe000u);
-          lo.w = v.w - __uint_as_float(__float_as_uint(v.w) & 0xffffe000u);
-        }
+        float4 lo;
+        lo.x = v.x - __uint_as_float(__float_as_uint(v.x) & 0xffffe000u);
+        lo.y = v.y - __uint_as_float(__float_as_uint(v.y) & 0xffffe000u);
+        lo.z = v.z - __uint_as_float(__float_as_uint(v.z) & 0xffffe000u);
+        lo.w = v.w - __uint_as_float(__float_as_uint(v.w) & 0xffffe000u);
         *reinterpret_cast<float4*>(lo_t + off) = lo;
       }
       fence_proxy_async();
@@ -1033,241 +632,11 @@ gemm_tc_tn_tma_kernel(const __grid_constant__ TmaDesc tmap_x, const __grid_const
   }
 }
 
-// ------------------------------------------------------------------ mode T kernel
-// C_partial[split][M tile rows][N] = sum over rows r in the split of X[r, m] * Y[r, n]
-// NBQ = float4 loads of Y per thread per K block (npad <= 32*NBQ).
-// MN = true keeps the operand tiles MN-major (rows of X / Y are stored as they arrive, 128-bit
-// shared-memory stores, UMMA descriptors with a_major = b_major = MN); MN = false transposes them
-// into K-major tiles with 32-bit stores.  npad must be a multiple of 32 when MN.
-
-template <int NBQ, bool MN>
-__global__ void __launch_bounds__(kThreads, (NBQ <= 2) ? 2 : 1)
-gemm_tc_tn_kernel(int64_t R, int M, int N, const float* __restrict__ x, int64_t ldx, const float* __restrict__ y,
-                  int64_t ldy, float* __restrict__ c, int64_t ldc, int64_t split_stride, int64_t rows_per_split,
-                  int npad, int tmem_cols, int vec_ok) {
-  extern __shared__ __align__(1024) uint8_t smem_raw[];
-  const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
-  Smem L;
-  smem_layout(npad, &L);
-  const uint32_t bar_mma[2] = {base + L.bars, base + L.bars + 8};
-  const uint32_t bar_acc = base + L.bars + 32;
-  const uint32_t tmem_slot = base + L.bars + 40;
-  uint8_t* gen = smem_raw + (base - smem_u32(smem_raw));
-
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  if (tid == 0) {
-    mbar_init(bar_mma[0], 1); mbar_init(bar_mma[1], 1);
-    mbar_init(bar_acc, 1);
-    fence_barrier_init();
-  }
-  if (tid < 32) {
-    __syncwarp();
-    tmem_alloc(tmem_slot, (uint32_t)tmem_cols);
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_d = *reinterpret_cast<volatile uint32_t*>(gen + L.bars + 40);
-  const uint32_t idesc = make_idesc(npad, MN);
-  const int ng = npad >> 5;
-
-  const int m0 = blockIdx.y * BM;
-  const int m_cols = min(BM, M - m0);          // valid rows of the C tile (= columns of X used)
-  const int64_t r_begin = (int64_t)blockIdx.x * rows_per_split;
-  const int64_t r_end = min(R, r_begin + rows_per_split);
-  const int nkb = (r_end > r_begin) ? (int)((r_end - r_begin + BKF - 1) / BKF) : 0;
-  const int a_q = (m_cols + 3) >> 2;  // float4 per X row inside this tile
-  const int b_q = (N + 3) >> 2;       // float4 per Y row
-
-  // Thread -> (reduction row k, float4 column q) of the K block.
-  //   MN-major tiles: lanes run along q, so a warp reads whole contiguous row segments (coalesced)
-  //     and each quarter-warp writes one full 128-byte shared-memory row (conflict free);
-  //   K-major tiles : lane <-> k, warps stride over q: the transposing STS.32 are conflict free.
-  int a_sh = 3, b_sh = 3;  // log2 of the float4 columns covered per row (power of two >= a_q / npad/4)
-  while ((1 << a_sh) < a_q) ++a_sh;
-  while ((1 << b_sh) < (npad >> 2)) ++b_sh;
-  auto item_a = [&](int j, int& k, int& q) -> bool {
-    if constexpr (MN) {
-      const int i = tid + kThreads * j;
-      k = i >> a_sh;
-      q = i & ((1 << a_sh) - 1);
-      return k < BKF;
-    } else {
-      k = lane;
-      q = warp + 8 * j;
-      return true;
-    }
-  };
-  auto item_b = [&](int j, int& k, int& q) -> bool {
-    if constexpr (MN) {
-      const int i = tid + kThreads * j;
-      k = i >> b_sh;
-      q = i & ((1 << b_sh) - 1);
-      return k < BKF;
-    } else {
-      k = lane;
-      q = warp + 8 * j;
-      return 4 * q < npad;
-    }
-  };
-  auto load_block = [&](int kb, float4 (&av)[4], float4 (&bv)[NBQ]) {
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-      int k, q;
-      av[j] = make_float4(0.f, 0.f, 0.f, 0.f);
-      if (item_a(j, k, q)) {
-        const int64_t r = r_begin + (int64_t)kb * BKF + k;
-        if (r < r_end && q < a_q) av[j] = __ldg(reinterpret_cast<const float4*>(x + r * ldx + m0 + 4 * q));
-      }
-    }
-#pragma unroll
-    for (int j = 0; j < NBQ; ++j) {
-      int k, q;
-      bv[j] = make_float4(0.f, 0.f, 0.f, 0.f);
-      if (item_b(j, k, q)) {
-        const int64_t r = r_begin + (int64_t)kb * BKF + k;
-        if (r < r_end && q < b_q) bv[j] = __ldg(reinterpret_cast<const float4*>(y + r * ldy + 4 * q));
-      }
-    }
-  };
-  // MN-major store: float4 q (elements 4q..4q+3) of reduction row k, groups-per-K-group gpk
-  auto store_mn = [&](uint32_t tile_hi, uint32_t tile_lo, int k, int q, int gpk, const float4& v) {
-    float4 hi, lo;
-    split_tf32(v.x, hi.x, lo.x); split_tf32(v.y, hi.y, lo.y);
-    split_tf32(v.z, hi.z, lo.z); split_tf32(v.w, hi.w, lo.w);
-    const uint32_t off = (uint32_t)(((q >> 3) + gpk * (k >> 2)) * 512 + (k & 3) * 128 +
-                                    (((((q & 7) >> 1) ^ (k & 3)) << 5) | ((q & 1) << 4)));
-    *reinterpret_cast<float4*>(gen + tile_hi + off) = hi;
-    *reinterpret_cast<float4*>(gen + tile_lo + off) = lo;
-  };
-  auto store_t = [&](uint32_t tile_hi, uint32_t tile_lo, int row4, const float4& v) {
-    const float e[4] = {v.x, v.y, v.z, v.w};
-#pragma unroll
-    for (int t = 0; t < 4; ++t) {
-      float hi, lo;
-      split_tf32(e[t], hi, lo);
-      const uint32_t off = sw128_off(row4 + t, lane);
-      *reinterpret_cast<float*>(gen + tile_hi + off) = hi;
-      *reinterpret_cast<float*>(gen + tile_lo + off) = lo;
-    }
-  };
-
-  // loads run two K blocks ahead of the transposing stores when the registers allow it (NBQ <= 2)
-  constexpr bool kDeep = NBQ <= 2;
-  float* cdst = c + (int64_t)blockIdx.x * split_stride;
-  uint32_t acc_parity = 0;
-  float4 av[4], bv[NBQ], a1[4], b1[NBQ], a2[kDeep ? 4 : 1], b2[kDeep ? NBQ : 1];
-  if (nkb > 0) load_block(0, av, bv);
-  if (nkb > 1) load_block(1, a1, b1);
-  for (int kb = 0; kb < nkb; ++kb) {
-    const int s = kb & 1;
-    const uint32_t use = (uint32_t)kb >> 1;
-    if constexpr (kDeep) {
-      if (kb + 2 < nkb) load_block(kb + 2, a2, b2);
-    }
-    if (use > 0) mbar_wait(bar_mma[s], (use - 1) & 1);
-    if constexpr (MN) {
-#pragma unroll
-      for (int j = 0; j < 4; ++j) {
-        int k, q;
-        if (item_a(j, k, q)) store_mn(L.a_hi[s], L.a_lo[s], k, q, 4, av[j]);
-      }
-#pragma unroll
-      for (int j = 0; j < NBQ; ++j) {
-        int k, q;
-        if (item_b(j, k, q)) store_mn(L.b_hi[s], L.b_lo[s], k, q, ng, bv[j]);
-      }
-    } else {
-#pragma unroll
-      for (int j = 0; j < 4; ++j) store_t(L.a_hi[s], L.a_lo[s], 4 * (warp + 8 * j), av[j]);
-#pragma unroll
-      for (int j = 0; j < NBQ; ++j)
-        if (4 * (warp + 8 * j) < npad) store_t(L.b_hi[s], L.b_lo[s], 4 * (warp + 8 * j), bv[j]);
-    }
-    fence_proxy_async();
-    __syncthreads();
-    // The tensor core adds into TMEM with truncation: after kTnDrainBlocks K blocks the accumulator is
-    // moved out (fp32 round-to-nearest adds into the partial tile in global memory, L2 resident) and
-    // restarted, like the rows kernel does, so that long reductions (2.4 M rows for the products-shaped
-    // dW) stay inside the fp32 tier's 1e-5.
-    const bool chunk_first = (kb % kTnDrainBlocks) == 0;
-    const bool chunk_last = (kb % kTnDrainBlocks) == kTnDrainBlocks - 1 || kb == nkb - 1;
-    if (tid == 0) {
-      tc_fence_after();
-      if constexpr (MN)
-        issue_kblock_mn(tmem_d, base + L.a_hi[s], base + L.a_lo[s], base + L.b_hi[s], base + L.b_lo[s], idesc, ng,
-                        chunk_first);
-      else
-        issue_kblock(tmem_d, base + L.a_hi[s], base + L.a_lo[s], base + L.b_hi[s], base + L.b_lo[s], idesc, chunk_first);
-      umma_commit(bar_mma[s]);
-      if (chunk_last) umma_commit(bar_acc);
-    }
-    if (chunk_last) {
-      mbar_wait(bar_acc, acc_parity);
-      acc_parity ^= 1u;
-      tc_fence_after();
-      epilogue_store(tmem_d, npad, cdst, ldc, m0, M, 0, N, vec_ok != 0, kb >= kTnDrainBlocks);
-      tc_fence_before();
-      __syncthreads();  // every warp has read its TMEM lanes before the next chunk overwrites them
-    }
-#pragma unroll
-    for (int j = 0; j < 4; ++j) av[j] = a1[j];
-#pragma unroll
-    for (int j = 0; j < NBQ; ++j) bv[j] = b1[j];
-    if constexpr (kDeep) {
-#pragma unroll
-      for (int j = 0; j < 4; ++j) a1[j] = a2[j];
-#pragma unroll
-      for (int j = 0; j < NBQ; ++j) b1[j] = b2[j];
-    } else {
-      if (kb + 2 < nkb) load_block(kb + 2, a1, b1);
-    }
-  }
-  if (nkb == 0) {
-    for (int i = tid; i < m_cols * N; i += kThreads) cdst[(int64_t)(m0 + i / N) * ldc + (i % N)] = 0.f;
-  }
-  __syncthreads();
-  if (tid < 32) {
-    __syncwarp();
-    tmem_dealloc(tmem_d, (uint32_t)tmem_cols);
-  }
-}
-
 inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
-inline int pad16(int64_t n) { return (int)(ceil_div(n, 16) * 16); }
 inline int tmem_cols_for(int npad) {
   int c = 32;
   while (c < npad) c <<= 1;
   return c;
-}
-
-struct RowsPlan { int npad, n_tiles, nkb; size_t img_floats; };
-RowsPlan rows_plan(int64_t n, int64_t k) {
-  RowsPlan p;
-  p.npad = n >= 256 ? 256 : pad16(n);
-  p.n_tiles = (int)ceil_div(n, p.npad);
-  p.nkb = (int)ceil_div(k, BKF);
-  p.img_floats = (size_t)p.n_tiles * p.nkb * p.npad * BKF;
-  return p;
-}
-
-// GCNB_ROWS_KERNEL=tma (default) | ws | sync; GCNB_TC_HI=rna makes the TMA kernel's splitters overwrite the raw
-// tile with cvt.rna values instead of letting the tensor core truncate the raw words
-int rows_kernel_choice() {  // 2 tma, 1 ws, 0 sync
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("GCNB_ROWS_KERNEL");
-    v = !e ? 2 : ((e[0] == 's' || e[0] == 'S') ? 0 : ((e[0] == 'w' || e[0] == 'W') ? 1 : 2));
-  }
-  return v;
-}
-int tma_hi_rna() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("GCNB_TC_HI");
-    v = (e && (e[0] == 'r' || e[0] == 'R')) ? 1 : 0;
-  }
-  return v;
 }
 
 // the 227 KB dynamic shared memory opt-in is a per-device attribute of the function: once per (kernel, device)
@@ -1384,31 +753,6 @@ TnTmaPlan tn_tma_plan(int64_t m, int64_t n, int64_t r) {
   return p;
 }
 
-// GCNB_TN_LAYOUT=k selects the transposing K-major variant of the tn kernel (default: MN-major)
-bool tn_use_mn() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("GCNB_TN_LAYOUT");
-    v = (e && (e[0] == 'k' || e[0] == 'K')) ? 0 : 1;
-  }
-  return v == 1;
-}
-
-struct TnPlan { int npad, m_tiles; int64_t splits, rows_per_split; };
-TnPlan tn_plan(int64_t m, int64_t n, int64_t r) {
-  TnPlan p;
-  p.npad = tn_use_mn() ? (int)(ceil_div(n, 32) * 32) : pad16(n);
-  p.m_tiles = (int)ceil_div(m, BM);
-  int64_t s = ceil_div(2 * kNumSMs, p.m_tiles);
-  const int64_t max_s = ceil_div(r, 4 * BKF);  // at least 4 K blocks per split
-  if (s > max_s) s = max_s;
-  if (s < 1) s = 1;
-  p.rows_per_split = ceil_div(ceil_div(r, s), BKF) * BKF;
-  p.splits = ceil_div(r, p.rows_per_split);
-  if (p.splits < 1) p.splits = 1;
-  return p;
-}
-
 }  // namespace
 
 // ------------------------------------------------------------------ host side
@@ -1416,176 +760,97 @@ bool gemm_tc_rows_eligible(int64_t m, int64_t n, int64_t k, const float* a, int6
                            const float* c, int64_t ldc) {
   (void)c; (void)ldc;
   return m > 0 && n > 0 && k > 0 && a_cs == 1 && (a_rs % 4 == 0) && (k % 4 == 0) && aligned16(a) &&
-         k <= (1 << 20) && n <= (1 << 20);
+         k <= (1 << 20) && n <= (1 << 20) && encode_tiled_fn() != nullptr;
 }
 
 size_t gemm_tc_rows_workspace_bytes(int64_t m, int64_t n, int64_t k) {
   (void)m;
-  const RowsPlan p = rows_plan(n, k);
-  const TmaPlan t = tma_plan(n, k);  // (pads N to 32: the larger image)
-  const size_t f = p.img_floats > t.img_floats ? p.img_floats : t.img_floats;
-  return 2 * f * sizeof(float) + 256;
+  return 2 * tma_plan(n, k).img_floats * sizeof(float) + 256;
 }
 
 int gemm_tc_rows_launch(int64_t m, int64_t n, int64_t k, const float* a, int64_t lda, const float* b, int64_t b_rs,
                         int64_t b_cs, float* c, int64_t ldc, void* ws, size_t ws_bytes, cudaStream_t st,
-                        const float* ep_bias, int ep_relu, bool* ep_done) {
+                        const float* ep_bias, int ep_relu) {
   GCNB_REQUIRE(ws != nullptr && ws_bytes >= gemm_tc_rows_workspace_bytes(m, n, k) && aligned16(ws),
                "gemm(tc rows): workspace too small or unaligned");
-  if (ep_done) *ep_done = false;  // only the TMA-fed kernel applies (bias, ReLU) itself; the caller finishes otherwise
-  if (rows_kernel_choice() == 2) {
-    const TmaPlan t = tma_plan(n, k);
+  const TmaPlan t = tma_plan(n, k);
+  GCNB_REQUIRE(t.ns >= 2, "gemm(tc rows): fewer than two operand stages fit in shared memory");
+  float* hi = reinterpret_cast<float*>(ws);
+  float* lo = hi + ((t.img_floats + 31) & ~(size_t)31);
+  int pg = (int)ceil_div((int64_t)t.img_floats, 256);
+  if (pg > 4 * kNumSMs) pg = 4 * kNumSMs;
+  const int vec = (ldc % 4 == 0) && aligned16(c);
+  const int tmem_cols = tmem_cols_for(2 * t.npad);
+  const bool pdl = pdl_enabled();  // opt-in: both kernels start while their predecessor drains (common.cuh)
+  if (pdl) {
+    GCNB_CUDA(launch_pdl(pack_b_kernel<true>, dim3((unsigned)pg), dim3(256), 0, st, k, n, t.npad, t.n_tiles, t.nkb, b,
+                         b_rs, b_cs, hi, lo));
+    GCNB_TRY(allow_big_smem(reinterpret_cast<const void*>(gemm_tc_rows_tma_kernel<true>), 2));
+  } else {
+    pack_b_kernel<false><<<pg, 256, 0, st>>>(k, n, t.npad, t.n_tiles, t.nkb, b, b_rs, b_cs, hi, lo);
+    GCNB_LAUNCH_CHECK();
+    GCNB_TRY(allow_big_smem(reinterpret_cast<const void*>(gemm_tc_rows_tma_kernel<false>), 0));
+  }
+  // The tensor map takes 32-bit row coordinates: a taller A runs in chunks of whole 128-row tiles, each with a map of
+  // its own.  A row's result does not depend on the chunk it is in.
+  const int64_t chunk_rows = (1ll << 31) - BM;
+  for (int64_t m0 = 0; m0 < m; m0 += chunk_rows) {
+    const int64_t mc = (m - m0 < chunk_rows) ? m - m0 : chunk_rows;
     TmaDesc tmap;
-    if (t.ns >= 2 && make_tmap_a(&tmap, a, m, k, lda)) {
-      float* hi = reinterpret_cast<float*>(ws);
-      float* lo = hi + ((t.img_floats + 31) & ~(size_t)31);
-      int pg = (int)ceil_div((int64_t)t.img_floats, 256);
-      if (pg > 4 * kNumSMs) pg = 4 * kNumSMs;
-      const int64_t mt = ceil_div(m, BM);
-      int64_t gx = kNumSMs / t.n_tiles;
-      if (gx < 1) gx = 1;
-      if (gx > mt) gx = mt;
-      const int vec = (ldc % 4 == 0) && aligned16(c);
-      if (pdl_enabled()) {  // opt-in: both kernels start while their predecessor drains (common.cuh)
-        GCNB_CUDA(launch_pdl(pack_b_kernel<true>, dim3((unsigned)pg), dim3(256), 0, st, k, n, t.npad, t.n_tiles, t.nkb, b,
-                             b_rs, b_cs, hi, lo));
-        GCNB_TRY(allow_big_smem(reinterpret_cast<const void*>(gemm_tc_rows_tma_kernel<true>), 2));
-        GCNB_CUDA(launch_pdl(gemm_tc_rows_tma_kernel<true>, dim3((unsigned)gx, (unsigned)t.n_tiles), dim3(kTmaThreads),
-                             t.smem, st, tmap, m, (int)n, (int)k, (const float*)hi, (const float*)lo, c, ldc, t.npad, t.nkb,
-                             (int)tmem_cols_for(2 * t.npad), vec, t.ns, t.b_resident, (int)tma_hi_rna(), ep_bias, ep_relu));
-        if (ep_done) *ep_done = true;
-        return GCNB_OK;
-      }
-      pack_b_kernel<false><<<pg, 256, 0, st>>>(k, n, t.npad, t.n_tiles, t.nkb, b, b_rs, b_cs, hi, lo);
+    GCNB_REQUIRE(make_tmap_a(&tmap, a + m0 * lda, mc, k, lda), "gemm(tc rows): tensor map encoding failed");
+    const int64_t mt = ceil_div(mc, BM);
+    int64_t gx = kNumSMs / t.n_tiles;
+    if (gx < 1) gx = 1;
+    if (gx > mt) gx = mt;
+    const dim3 grid((unsigned)gx, (unsigned)t.n_tiles);
+    if (pdl) {
+      GCNB_CUDA(launch_pdl(gemm_tc_rows_tma_kernel<true>, grid, dim3(kTmaThreads), t.smem, st, tmap, mc, (int)n, (int)k,
+                           (const float*)hi, (const float*)lo, c + m0 * ldc, ldc, t.npad, t.nkb, tmem_cols, vec, t.ns,
+                           t.b_resident, ep_bias, ep_relu));
+    } else {
+      gemm_tc_rows_tma_kernel<false><<<grid, kTmaThreads, t.smem, st>>>(tmap, mc, (int)n, (int)k, hi, lo, c + m0 * ldc,
+                                                                       ldc, t.npad, t.nkb, tmem_cols, vec, t.ns,
+                                                                       t.b_resident, ep_bias, ep_relu);
       GCNB_LAUNCH_CHECK();
-      GCNB_TRY(allow_big_smem(reinterpret_cast<const void*>(gemm_tc_rows_tma_kernel<false>), 0));
-      gemm_tc_rows_tma_kernel<false><<<dim3((unsigned)gx, (unsigned)t.n_tiles), kTmaThreads, t.smem, st>>>(
-          tmap, m, (int)n, (int)k, hi, lo, c, ldc, t.npad, t.nkb, tmem_cols_for(2 * t.npad), vec, t.ns, t.b_resident,
-          tma_hi_rna(), ep_bias, ep_relu);
-      GCNB_LAUNCH_CHECK();
-      if (ep_done) *ep_done = true;
-      return GCNB_OK;
     }
   }
-  const RowsPlan p = rows_plan(n, k);
-  float* img_hi = reinterpret_cast<float*>(ws);
-  float* img_lo = img_hi + ((p.img_floats + 31) & ~(size_t)31);
-  GCNB_REQUIRE((size_t)((char*)(img_lo + p.img_floats) - (char*)ws) <= ws_bytes, "gemm(tc rows): workspace layout");
-  const int64_t total = (int64_t)p.img_floats;
-  int pgrid = (int)ceil_div(total, 256);
-  if (pgrid > 4 * kNumSMs) pgrid = 4 * kNumSMs;
-  pack_b_kernel<false><<<pgrid, 256, 0, st>>>(k, n, p.npad, p.n_tiles, p.nkb, b, b_rs, b_cs, img_hi, img_lo);
-  GCNB_LAUNCH_CHECK();
-  Smem L;
-  // keep the packed B resident when it costs no occupancy (<= 40 KB on top of the 64 KB of A stages)
-  const int b_resident = ((size_t)p.nkb * 2 * p.npad * 128 <= 40 * 1024) ? 1 : 0;
-  const uint32_t smem = smem_layout(p.npad, &L, b_resident ? p.nkb : 2) + 1024;
-  // (the opt-in is per device and cheap: set it before every launch rather than remember it per process)
-  GCNB_CUDA(cudaFuncSetAttribute(gemm_tc_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-  const int64_t m_tiles = ceil_div(m, BM);
-  const int vec_ok_ = (ldc % 4 == 0) && aligned16(c) && (p.npad % 4 == 0);
-  if (b_resident && rows_kernel_choice() >= 1) {
-    // warp-specialised pipeline: as many 32 KB operand stages as fit beside the resident B (<= 4)
-    const size_t b_total = (size_t)p.nkb * 2 * p.npad * 128;
-    int ns = (int)((200 * 1024 - b_total) / (2 * kTileBytes));
-    if (ns > 4) ns = 4;
-    const uint32_t smem_ws = (uint32_t)(ns * 2 * kTileBytes + ((b_total + 1023) & ~(size_t)1023) + 1024 + 1024);
-    GCNB_CUDA(cudaFuncSetAttribute(gemm_tc_rows_ws_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-    int64_t gxw = kNumSMs / p.n_tiles;
-    if (gxw < 1) gxw = 1;
-    if (gxw > m_tiles) gxw = m_tiles;
-    dim3 gridw((unsigned)gxw, (unsigned)p.n_tiles);
-    gemm_tc_rows_ws_kernel<<<gridw, kWsThreads, smem_ws, st>>>(m, (int)n, (int)k, a, lda, img_hi, img_lo, c, ldc, p.npad,
-                                                              p.nkb, tmem_cols_for(2 * p.npad), vec_ok_, ns);
-    GCNB_LAUNCH_CHECK();
-    return GCNB_OK;
-  }
-  const int ctas_per_sm = (smem <= 110 * 1024) ? 2 : 1;
-  int64_t gx = (int64_t)kNumSMs * ctas_per_sm / p.n_tiles;
-  if (gx < 1) gx = 1;
-  if (gx > m_tiles) gx = m_tiles;
-  dim3 grid((unsigned)gx, (unsigned)p.n_tiles);
-  const int vec_ok = (ldc % 4 == 0) && aligned16(c) && (p.npad % 4 == 0);
-  gemm_tc_rows_kernel<<<grid, kThreads, smem, st>>>(m, (int)n, (int)k, a, lda, img_hi, img_lo, c, ldc, p.npad, p.nkb,
-                                                    tmem_cols_for(p.npad), vec_ok, b_resident);
-  GCNB_LAUNCH_CHECK();
   return GCNB_OK;
 }
 
-// narrow "rows" products with K >= 32 measure faster on the TMA-fed tensor-core kernel than on the CUDA-core
-// skinny kernel (CBG 64->32 X W: 23.1 vs 26.6 us in the step's graph; 8->32: 16.6 vs 12.3)
-bool gemm_tc_rows_beats_skinny(int64_t k) { return rows_kernel_choice() == 2 && k >= 32 && encode_tiled_fn() != nullptr; }
+// narrow "rows" products with K >= 32 measure faster on the tensor-core kernel than on the CUDA-core skinny kernel
+// (CBG 64->32 X W: 23.1 vs 26.6 us in the step's graph; 8->32: 16.6 vs 12.3)
+bool gemm_tc_rows_beats_skinny(int64_t k) { return k >= 32 && encode_tiled_fn() != nullptr; }
 
-// dW-shaped product: C[M,N] = sum_r X[r, 0:M]^T Y[r, 0:N]
-// padded = every row of x / y is readable (and finite) up to the next multiple of 4 columns
-bool gemm_tc_tn_eligible(int64_t m, int64_t n, int64_t r, const float* x, int64_t ldx, const float* y, int64_t ldy,
-                         bool padded) {
-  // the TMA-fed kernel zero-fills past the widths itself; the register-fed one reads whole float4s
-  const bool tma = rows_kernel_choice() == 2 && tn_use_mn() && encode_tiled_fn() != nullptr;
-  const bool widths_ok = tma ? true
-                             : (padded ? (ldx >= ceil_div(m, 4) * 4 && ldy >= ceil_div(n, 4) * 4) : (m % 4 == 0 && n % 4 == 0));
-  return m > 0 && n > 0 && r > 0 && n <= 256 && (ldx % 4 == 0) && (ldy % 4 == 0) && widths_ok && aligned16(x) &&
-         aligned16(y);
+// dW-shaped product: C[M,N] = sum_r X[r, 0:M]^T Y[r, 0:N].  The kernel zero-fills past the widths itself; the
+// tensor maps take 32-bit coordinates.
+bool gemm_tc_tn_eligible(int64_t m, int64_t n, int64_t r, const float* x, int64_t ldx, const float* y, int64_t ldy) {
+  return m > 0 && n > 0 && r > 0 && n <= 256 && m < (1ll << 31) && r < (1ll << 31) && (ldx % 4 == 0) &&
+         (ldy % 4 == 0) && aligned16(x) && aligned16(y) && encode_tiled_fn() != nullptr;
 }
 
 size_t gemm_tc_tn_workspace_bytes(int64_t m, int64_t n, int64_t r) {
-  const TnPlan p = tn_plan(m, n, r);
-  return p.splits > 1 ? (size_t)p.splits * (size_t)m * (size_t)n * sizeof(float) : 0;
+  const TnTmaPlan t = tn_tma_plan(m, n, r);
+  return t.splits > 1 ? (size_t)t.splits * (size_t)m * (size_t)n * sizeof(float) : 0;
 }
 
 int gemm_tc_tn_launch(int64_t m, int64_t n, int64_t r, const float* x, int64_t ldx, const float* y, int64_t ldy,
                       float* c, int64_t ldc, void* ws, size_t ws_bytes, cudaStream_t st) {
-  const TnPlan p = tn_plan(m, n, r);
+  const TnTmaPlan t = tn_tma_plan(m, n, r);
   const size_t need = gemm_tc_tn_workspace_bytes(m, n, r);
   GCNB_REQUIRE(need == 0 || (ws != nullptr && ws_bytes >= need && aligned16(ws)), "gemm(tc tn): workspace too small");
-  if (rows_kernel_choice() == 2 && tn_use_mn() && n <= 256) {
-    const TnTmaPlan t = tn_tma_plan(m, n, r);
-    TmaDesc tx, ty;
-    const size_t need_t = t.splits > 1 ? (size_t)t.splits * (size_t)m * (size_t)n * sizeof(float) : 0;
-    if (t.ns >= 2 && need_t <= ws_bytes && make_tmap_mn(&tx, x, r, m, ldx) && make_tmap_mn(&ty, y, r, n, ldy)) {
-      float* dst_t = (t.splits > 1) ? reinterpret_cast<float*>(ws) : c;
-      const int64_t ld_t = (t.splits > 1) ? n : ldc;
-      const int64_t stride_t = (t.splits > 1) ? m * n : 0;
-      const int vec = (ld_t % 4 == 0) && aligned16(dst_t);
-      GCNB_TRY(allow_big_smem(reinterpret_cast<const void*>(gemm_tc_tn_tma_kernel), 1));
-      gemm_tc_tn_tma_kernel<<<dim3((unsigned)t.splits, (unsigned)t.m_tiles), kTmaThreads, t.smem, st>>>(
-          tx, ty, r, (int)m, (int)n, dst_t, ld_t, stride_t, t.rows_per_split, t.npad, tmem_cols_for(2 * t.npad), vec, t.ns);
-      GCNB_LAUNCH_CHECK();
-      if (t.splits > 1) GCNB_TRY(reduce_partials_launch(m, n, (int)t.splits, dst_t, c, ldc, st));
-      return GCNB_OK;
-    }
-  }
-  GCNB_REQUIRE(ldx >= ceil_div(m, 4) * 4 && ldy >= ceil_div(n, 4) * 4,
-               "gemm(tc tn): rows must be readable up to the next multiple of 4 columns without the TMA kernel");
-  Smem L;
-  const uint32_t smem = smem_layout(p.npad, &L) + 1024;
-  float* dst = (p.splits > 1) ? reinterpret_cast<float*>(ws) : c;
-  const int64_t dst_ld = (p.splits > 1) ? n : ldc;
-  const int64_t stride = (p.splits > 1) ? m * n : 0;
-  const int vec_ok = (dst_ld % 4 == 0) && aligned16(dst);
-  dim3 grid((unsigned)p.splits, (unsigned)p.m_tiles);
-#define GCNB_TN_LAUNCH(NBQ_, MN_)                                                                                  \
-  do {                                                                                                             \
-    GCNB_CUDA(cudaFuncSetAttribute(gemm_tc_tn_kernel<NBQ_, MN_>, cudaFuncAttributeMaxDynamicSharedMemorySize,      \
-                                   227 * 1024));                                                                   \
-    gemm_tc_tn_kernel<NBQ_, MN_><<<grid, kThreads, smem, st>>>(r, (int)m, (int)n, x, ldx, y, ldy, dst, dst_ld,     \
-                                                               stride, p.rows_per_split, p.npad,                   \
-                                                               tmem_cols_for(p.npad), vec_ok);                     \
-  } while (0)
-  if (tn_use_mn()) {
-    if (p.npad <= 32) GCNB_TN_LAUNCH(1, true);
-    else if (p.npad <= 64) GCNB_TN_LAUNCH(2, true);
-    else if (p.npad <= 128) GCNB_TN_LAUNCH(4, true);
-    else GCNB_TN_LAUNCH(8, true);
-  } else {
-    if (p.npad <= 32) GCNB_TN_LAUNCH(1, false);
-    else if (p.npad <= 64) GCNB_TN_LAUNCH(2, false);
-    else if (p.npad <= 128) GCNB_TN_LAUNCH(4, false);
-    else GCNB_TN_LAUNCH(8, false);
-  }
-#undef GCNB_TN_LAUNCH
+  GCNB_REQUIRE(t.ns >= 2, "gemm(tc tn): fewer than two operand stages fit in shared memory");
+  TmaDesc tx, ty;
+  GCNB_REQUIRE(make_tmap_mn(&tx, x, r, m, ldx) && make_tmap_mn(&ty, y, r, n, ldy),
+               "gemm(tc tn): tensor map encoding failed");
+  float* dst = (t.splits > 1) ? reinterpret_cast<float*>(ws) : c;
+  const int64_t ld = (t.splits > 1) ? n : ldc;
+  const int64_t stride = (t.splits > 1) ? m * n : 0;
+  const int vec = (ld % 4 == 0) && aligned16(dst);
+  GCNB_TRY(allow_big_smem(reinterpret_cast<const void*>(gemm_tc_tn_tma_kernel), 1));
+  gemm_tc_tn_tma_kernel<<<dim3((unsigned)t.splits, (unsigned)t.m_tiles), kTmaThreads, t.smem, st>>>(
+      tx, ty, r, (int)m, (int)n, dst, ld, stride, t.rows_per_split, t.npad, tmem_cols_for(2 * t.npad), vec, t.ns);
   GCNB_LAUNCH_CHECK();
-  if (p.splits > 1) GCNB_TRY(reduce_partials_launch(m, n, (int)p.splits, dst, c, ldc, st));
+  if (t.splits > 1) GCNB_TRY(reduce_partials_launch(m, n, (int)t.splits, dst, c, ldc, st));
   return GCNB_OK;
 }
 

@@ -1,6 +1,5 @@
 """Accuracy (vs fp64) and time of the tcgen05 "rows" product C = A[M,K] B[K,N] on the layer shapes of the
-BASELINE configs, for whichever kernel the environment selects (GCNB_ROWS_KERNEL = tma | ws | sync,
-GCNB_TC_HI = trunc | rna).  Run on the GPU box:  python tools/gemm_rows_probe.py [tag]"""
+BASELINE configs.  Run on the GPU box:  python tools/gemm_rows_probe.py [tag]"""
 import os
 import sys
 
@@ -11,7 +10,7 @@ import pygcn_b200 as P
 
 dev = torch.device("cuda:0")
 torch.manual_seed(0)
-tag = sys.argv[1] if len(sys.argv) > 1 else "%s/%s" % (os.environ.get("GCNB_ROWS_KERNEL", "tma"), os.environ.get("GCNB_TC_HI", "trunc"))
+tag = sys.argv[1] if len(sys.argv) > 1 else "tcgen05"
 
 
 def timeit(fn, n=10):

@@ -11,11 +11,10 @@ import pygcn_b200 as P
 from time_step import dev, graph_time
 
 torch.manual_seed(0)
-tag = "rows=%s hi=%s" % (os.environ.get("GCNB_ROWS_KERNEL", "tma"), os.environ.get("GCNB_TC_HI", "trunc"))
 tiny = torch.zeros(32, 4, device=dev)
 w4 = torch.zeros(4, 4, device=dev)
 t0 = graph_time(lambda: P.mm(tiny, w4, precision="fp32"))
-print("[%s] graph replay of one tiny kernel: %.1f us (subtract from the numbers below)" % (tag, t0))
+print("graph replay of one tiny kernel: %.1f us (subtract from the numbers below)" % t0)
 for (m, k, n, what) in [(100000, 64, 32, "CBG"), (100000, 32, 32, "fork-like 32->32"), (100000, 8, 32, "fork 8->32"),
                         (233000, 604, 256, "Reddit"), (1000000, 128, 128, "papers (1M rows)")]:
     x = torch.randn(m, k, device=dev)
