@@ -190,9 +190,10 @@ int pad_copy_launch(int64_t n_rows, int64_t w, const float* src, int64_t ld_src,
 
 int bias_act_launch(int64_t n_rows, int64_t f, float* out, int64_t ldo, const Epilogue& ep, cudaStream_t stream);
 
-// extra_row != nullptr: every part holds m + 1 rows and the sum of row m goes to extra_row[0:n]
+// xout != nullptr: also xout[0:n] = the sum over parts of the fp64 xpart[n_parts][n], rounded to fp32 once (column
+// sums); m may then be 0
 int reduce_partials_launch(int64_t m, int64_t n, int n_parts, const float* partial, float* out,
-                           int64_t ldo, cudaStream_t stream, float* extra_row = nullptr);
+                           int64_t ldo, cudaStream_t stream, const double* xpart = nullptr, float* xout = nullptr);
 
 }  // namespace gcnb
 

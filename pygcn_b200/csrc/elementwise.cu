@@ -10,15 +10,16 @@ namespace {
 constexpr int kThreads = 256;
 constexpr int kMaxBlocks = 4 * kNumSMs;
 
-// Phase 1: block b reduces rows [b*rows_per_block, ...) -> partial[b][0:f]
+// Phase 1: block b reduces rows [b*rows_per_block, ...) -> partial[b][0:f] (fp64)
 __global__ void __launch_bounds__(kThreads)
 colsum_partial_kernel(int64_t n_rows, int f, int cw, int64_t rows_per_block,
                       const float* __restrict__ g, int64_t ldg, const float* __restrict__ y,
                       int64_t ldy, float* __restrict__ gm, int64_t ldgm,
-                      float* __restrict__ partial, const uint8_t* __restrict__ mask, int64_t ld_mask,
+                      double* __restrict__ partial, const uint8_t* __restrict__ mask, int64_t ld_mask,
                       float mask_scale) {
-  // (fp64 accumulators: a column of the upstream gradient is 10^6 terms of either sign that cancel to ~sqrt(N) of
-  // their mass; the kernel is memory-bound, the DADDs are free, and db then carries fp32 rounding of the RESULT only)
+  // (fp64 accumulators AND fp64 block partials: a column of the upstream gradient is 10^6 terms of either sign that
+  // cancel to ~sqrt(N) of their mass; the kernel is memory-bound, the DADDs are free, and db then carries fp32
+  // rounding of the RESULT only -- a partial rounded to fp32 would lose what the other blocks' partials cancel)
   __shared__ double red[kThreads];
   const int tx = threadIdx.x % cw;  // column lane
   const int ty = threadIdx.x / cw;  // row lane
@@ -64,7 +65,7 @@ colsum_partial_kernel(int64_t n_rows, int f, int cw, int64_t rows_per_block,
     if (ty == 0 && j < f) {
       double s = 0.0;
       for (int t = 0; t < rl; ++t) s += red[t * cw + tx];
-      partial[(int64_t)blockIdx.x * f + j] = (float)s;
+      partial[(int64_t)blockIdx.x * f + j] = s;
     }
     __syncthreads();
   }
@@ -77,9 +78,9 @@ colsum_partial_kernel(int64_t n_rows, int f, int cw, int64_t rows_per_block,
 __global__ void __launch_bounds__(kThreads)
 colsum_vec_kernel(int64_t n_rows, int f4, int cw, int64_t rows_per_block, const float4* __restrict__ g, int64_t ldg4,
                   const float4* __restrict__ y, int64_t ldy4, float4* __restrict__ gm, int64_t ldgm4,
-                  float4* __restrict__ partial, unsigned int* __restrict__ ticket, float* __restrict__ out,
+                  double2* __restrict__ partial, unsigned int* __restrict__ ticket, float* __restrict__ out,
                   const uchar4* __restrict__ mask, int64_t ld_mask4, float mask_scale) {
-  __shared__ double red[kThreads][4];  // fp64 accumulation, see colsum_partial_kernel
+  __shared__ double red[kThreads][4];  // fp64 accumulation and fp64 partials, see colsum_partial_kernel
   __shared__ bool is_last;
   const int tx = threadIdx.x % cw;  // float4 column chunk
   const int ty = threadIdx.x / cw;  // row lane
@@ -124,7 +125,8 @@ colsum_vec_kernel(int64_t n_rows, int f4, int cw, int64_t rows_per_block, const 
     for (int t = 0; t < rl; ++t)
 #pragma unroll
       for (int c = 0; c < 4; ++c) s[c] += red[t * cw + tx][c];
-    partial[(int64_t)blockIdx.x * f4 + tx] = make_float4((float)s[0], (float)s[1], (float)s[2], (float)s[3]);
+    partial[2 * ((int64_t)blockIdx.x * f4 + tx)] = make_double2(s[0], s[1]);
+    partial[2 * ((int64_t)blockIdx.x * f4 + tx) + 1] = make_double2(s[2], s[3]);
   }
   __threadfence();
   __syncthreads();
@@ -137,8 +139,8 @@ colsum_vec_kernel(int64_t n_rows, int f4, int cw, int64_t rows_per_block, const 
   for (int c = 0; c < 4; ++c) acc[c] = 0.0;
   if (tx < f4) {
     for (int b = ty; b < (int)gridDim.x; b += rl) {
-      const float4 v = partial[(int64_t)b * f4 + tx];
-      acc[0] += v.x; acc[1] += v.y; acc[2] += v.z; acc[3] += v.w;
+      const double2 v = partial[2 * ((int64_t)b * f4 + tx)], w = partial[2 * ((int64_t)b * f4 + tx) + 1];
+      acc[0] += v.x; acc[1] += v.y; acc[2] += w.x; acc[3] += w.y;
     }
   }
 #pragma unroll
@@ -153,36 +155,51 @@ colsum_vec_kernel(int64_t n_rows, int f4, int cw, int64_t rows_per_block, const 
   }
 }
 
-// out[i] = sum over parts of partial[s][i]: 32 outputs x 8 part-lanes per CTA, fixed-order tree.
+// Lane ty of a part sum adds parts ty, ty + lanes, ...: four loads in flight, added in a fixed order (T = float for
+// the tiles of a split product, double for the column-sum partials).
+template <typename T, int kLanes>
+__device__ __forceinline__ T sum_parts(const T* __restrict__ p, int64_t stride, int64_t i, int n_parts, int ty) {
+  T a0 = 0, a1 = 0, a2 = 0, a3 = 0;
+  int s = ty;
+  for (; s + 3 * kLanes < n_parts; s += 4 * kLanes) {
+    a0 += p[(int64_t)s * stride + i];
+    a1 += p[(int64_t)(s + kLanes) * stride + i];
+    a2 += p[(int64_t)(s + 2 * kLanes) * stride + i];
+    a3 += p[(int64_t)(s + 3 * kLanes) * stride + i];
+  }
+  for (; s < n_parts; s += kLanes) a0 += p[(int64_t)s * stride + i];
+  return (a0 + a1) + (a2 + a3);
+}
+
+// out[i / n, i % n] = sum over parts of the fp32 partial[s][i] for i < m * n, and -- when xout is given -- one more
+// row: xout[j] = sum over parts of the fp64 xpart[s][j], rounded to fp32 once (column sums).  32 outputs x 8
+// part-lanes per CTA, fixed-order tree (an fp32 lane sum goes through the fp64 shared array unchanged).
 __global__ void __launch_bounds__(kThreads)
 reduce_partials_kernel(int64_t total, int64_t n, int n_parts, const float* __restrict__ partial,
-                       float* __restrict__ out, int64_t ldo, int64_t m, float* __restrict__ extra_row) {
-  __shared__ float red[8][33];
+                       float* __restrict__ out, int64_t ldo, int64_t m, const double* __restrict__ xpart,
+                       float* __restrict__ xout) {
+  __shared__ double red[8][33];
   const int tx = threadIdx.x & 31;
   const int ty = threadIdx.x >> 5;
   const int64_t i = (int64_t)blockIdx.x * 32 + tx;
-  float acc = 0.f;
-  if (i < total) {
-    // lane ty owns parts ty, ty+8, ...: four loads in flight, added in a fixed order
-    float a0 = 0.f, a1 = 0.f, a2 = 0.f, a3 = 0.f;
-    int s = ty;
-    for (; s + 24 < n_parts; s += 32) {
-      a0 += partial[(int64_t)s * total + i];
-      a1 += partial[(int64_t)(s + 8) * total + i];
-      a2 += partial[(int64_t)(s + 16) * total + i];
-      a3 += partial[(int64_t)(s + 24) * total + i];
-    }
-    for (; s < n_parts; s += 8) a0 += partial[(int64_t)s * total + i];
-    acc = (a0 + a1) + (a2 + a3);
-  }
+  const int64_t mn = m * n;
+  double acc = 0.0;
+  if (i < total) acc = (i < mn) ? (double)sum_parts<float, 8>(partial, mn, i, n_parts, ty)
+                                : sum_parts<double, 8>(xpart, n, i - mn, n_parts, ty);
   red[ty][tx] = acc;
   __syncthreads();
   if (ty == 0 && i < total) {
-    float v = 0.f;
+    if (i < mn) {
+      float v = 0.f;
 #pragma unroll
-    for (int t = 0; t < 8; ++t) v += red[t][tx];
-    if (i / n < m) out[(i / n) * ldo + (i % n)] = v;
-    else extra_row[i % n] = v;  // row m of every part: the fused column sum
+      for (int t = 0; t < 8; ++t) v += (float)red[t][tx];
+      out[(i / n) * ldo + (i % n)] = v;
+    } else {
+      double v = 0.0;
+#pragma unroll
+      for (int t = 0; t < 8; ++t) v += red[t][tx];
+      xout[i - mn] = (float)v;
+    }
   }
 }
 
@@ -192,8 +209,10 @@ reduce_partials_kernel(int64_t total, int64_t n, int n_parts, const float* __res
 template <bool PDL>  // (the programmatic-dependent-launch instantiation, common.cuh)
 __global__ void __launch_bounds__(kThreads)
 reduce_partials_vec_kernel(int64_t total4, int64_t n4, int n_parts, const float4* __restrict__ partial,
-                           float* __restrict__ out, int64_t ldo, int64_t m, float* __restrict__ extra_row) {
+                           float* __restrict__ out, int64_t ldo, int64_t m, const double2* __restrict__ xpart,
+                           float* __restrict__ xout) {
   __shared__ float4 red[32][8];
+  __shared__ double2 xred[32][8][2];
   if constexpr (PDL) {
     pdl_launch_dependents();
     pdl_wait();  // the partial tiles are the previous kernel's output
@@ -201,35 +220,49 @@ reduce_partials_vec_kernel(int64_t total4, int64_t n4, int n_parts, const float4
   const int tx = threadIdx.x & 7;
   const int ty = threadIdx.x >> 3;
   const int64_t i = (int64_t)blockIdx.x * 8 + tx;
-  float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
-  if (i < total4) {
+  const int64_t mn4 = m * n4;
+  if (i < mn4) {  // (warp-uniform except in the one warp that straddles row m)
+    float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
     int s = ty;
     for (; s + 96 < n_parts; s += 128) {
-      const float4 v0 = __ldg(partial + (int64_t)s * total4 + i);
-      const float4 v1 = __ldg(partial + (int64_t)(s + 32) * total4 + i);
-      const float4 v2 = __ldg(partial + (int64_t)(s + 64) * total4 + i);
-      const float4 v3 = __ldg(partial + (int64_t)(s + 96) * total4 + i);
+      const float4 v0 = __ldg(partial + (int64_t)s * mn4 + i);
+      const float4 v1 = __ldg(partial + (int64_t)(s + 32) * mn4 + i);
+      const float4 v2 = __ldg(partial + (int64_t)(s + 64) * mn4 + i);
+      const float4 v3 = __ldg(partial + (int64_t)(s + 96) * mn4 + i);
       acc.x = (((acc.x + v0.x) + v1.x) + v2.x) + v3.x;
       acc.y = (((acc.y + v0.y) + v1.y) + v2.y) + v3.y;
       acc.z = (((acc.z + v0.z) + v1.z) + v2.z) + v3.z;
       acc.w = (((acc.w + v0.w) + v1.w) + v2.w) + v3.w;
     }
     for (; s < n_parts; s += 32) {
-      const float4 v = __ldg(partial + (int64_t)s * total4 + i);
+      const float4 v = __ldg(partial + (int64_t)s * mn4 + i);
       acc.x += v.x; acc.y += v.y; acc.z += v.z; acc.w += v.w;
     }
+    red[ty][tx] = acc;
+  } else if (i < total4) {  // the fp64 column-sum row
+    double a[4] = {0.0, 0.0, 0.0, 0.0};
+    for (int s = ty; s < n_parts; s += 32) {
+      const double2 v = __ldg(xpart + 2 * ((int64_t)s * n4 + (i - mn4))), w = __ldg(xpart + 2 * ((int64_t)s * n4 + (i - mn4)) + 1);
+      a[0] += v.x; a[1] += v.y; a[2] += w.x; a[3] += w.y;
+    }
+    xred[ty][tx][0] = make_double2(a[0], a[1]);
+    xred[ty][tx][1] = make_double2(a[2], a[3]);
   }
-  red[ty][tx] = acc;
   __syncthreads();
-  if (ty == 0 && i < total4) {
+  if (ty == 0 && i < mn4) {
     float4 v = red[0][tx];
 #pragma unroll
     for (int t = 1; t < 32; ++t) {
       const float4 r = red[t][tx];
       v.x += r.x; v.y += r.y; v.z += r.z; v.w += r.w;
     }
-    float* dst = (i / n4 < m) ? out + (i / n4) * ldo + 4 * (i % n4) : extra_row + 4 * (i % n4);
-    *reinterpret_cast<float4*>(dst) = v;
+    *reinterpret_cast<float4*>(out + (i / n4) * ldo + 4 * (i % n4)) = v;
+  } else if (ty == 0 && i < total4) {
+    double a[4] = {0.0, 0.0, 0.0, 0.0};
+    for (int t = 0; t < 32; ++t) {
+      a[0] += xred[t][tx][0].x; a[1] += xred[t][tx][0].y; a[2] += xred[t][tx][1].x; a[3] += xred[t][tx][1].y;
+    }
+    *reinterpret_cast<float4*>(xout + 4 * (i - mn4)) = make_float4((float)a[0], (float)a[1], (float)a[2], (float)a[3]);
   }
 }
 
@@ -278,8 +311,8 @@ int colsum_blocks(int64_t n_rows) {
 }  // namespace
 
 size_t colsum_workspace_bytes(int64_t n_rows, int64_t f) {
-  // partials [blocks][f] (16-byte aligned rows) + the arrival ticket of the single-launch variant
-  return (size_t)colsum_blocks(n_rows) * (size_t)(ceil_div(f, 4) * 4) * sizeof(float) + 256;
+  // fp64 partials [blocks][f] (32-byte aligned rows) + the arrival ticket of the single-launch variant
+  return (size_t)colsum_blocks(n_rows) * (size_t)(ceil_div(f, 4) * 4) * sizeof(double) + 256;
 }
 
 int colsum_launch(int64_t n_rows, int64_t f, const float* g, int64_t ldg, const float* y,
@@ -299,6 +332,7 @@ int colsum_launch(int64_t n_rows, int64_t f, const float* g, int64_t ldg, const 
   const int nb = colsum_blocks(n_rows);
   const size_t need = colsum_workspace_bytes(n_rows, f);
   GCNB_REQUIRE(ws != nullptr && ws_bytes >= need, "colsum: workspace too small (%zu < %zu)", ws_bytes, need);
+  GCNB_REQUIRE((reinterpret_cast<uintptr_t>(ws) & 7u) == 0, "colsum: workspace not 8-byte aligned (fp64 partials)");
   const int64_t rows_per_block = ceil_div(n_rows, nb);
   auto al16 = [](const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; };
   const bool vec = f % 4 == 0 && f <= 4 * kThreads && al16(g) && ldg % 4 == 0 && al16(out) && al16(ws) &&
@@ -312,7 +346,7 @@ int colsum_launch(int64_t n_rows, int64_t f, const float* g, int64_t ldg, const 
     GCNB_CUDA(cudaMemsetAsync(ticket, 0, sizeof(unsigned int), st));
     colsum_vec_kernel<<<nb, kThreads, 0, st>>>(
         n_rows, f4, cw4, rows_per_block, reinterpret_cast<const float4*>(g), ldg / 4, reinterpret_cast<const float4*>(y),
-        ldy / 4, reinterpret_cast<float4*>(gm), ldgm / 4, reinterpret_cast<float4*>(ws), ticket, out,
+        ldy / 4, reinterpret_cast<float4*>(gm), ldgm / 4, reinterpret_cast<double2*>(ws), ticket, out,
         reinterpret_cast<const uchar4*>(mask), ld_mask / 4, mask_scale);
     GCNB_LAUNCH_CHECK();
     return GCNB_OK;
@@ -320,9 +354,9 @@ int colsum_launch(int64_t n_rows, int64_t f, const float* g, int64_t ldg, const 
   int cw = 32;
   while (cw < f && cw < kThreads) cw <<= 1;
   colsum_partial_kernel<<<nb, kThreads, 0, st>>>(n_rows, (int)f, cw, rows_per_block, g, ldg, y, ldy, gm,
-                                                 ldgm, reinterpret_cast<float*>(ws), mask, ld_mask, mask_scale);
+                                                 ldgm, reinterpret_cast<double*>(ws), mask, ld_mask, mask_scale);
   GCNB_LAUNCH_CHECK();
-  return reduce_partials_launch(1, f, nb, reinterpret_cast<const float*>(ws), out, f, st);
+  return reduce_partials_launch(0, f, nb, nullptr, nullptr, 0, st, reinterpret_cast<const double*>(ws), out);
 }
 
 int pad_copy_launch(int64_t n_rows, int64_t w, const float* src, int64_t ld_src, float* dst, int64_t ld_dst,
@@ -390,23 +424,25 @@ int bias_act_launch(int64_t n_rows, int64_t f, float* out, int64_t ldo, const Ep
 }
 
 int reduce_partials_launch(int64_t m, int64_t n, int n_parts, const float* partial, float* out,
-                           int64_t ldo, cudaStream_t st, float* extra_row) {
-  const int64_t total = (m + (extra_row ? 1 : 0)) * n;
+                           int64_t ldo, cudaStream_t st, const double* xpart, float* xout) {
+  const int64_t total = (m + (xout ? 1 : 0)) * n;
   if (total == 0) return GCNB_OK;
-  if (n_parts >= 16 && n % 4 == 0 && ldo % 4 == 0 && (reinterpret_cast<uintptr_t>(partial) & 15u) == 0 &&
-      (reinterpret_cast<uintptr_t>(out) & 15u) == 0 && (reinterpret_cast<uintptr_t>(extra_row) & 15u) == 0) {
+  auto al16 = [](const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; };
+  if (n_parts >= 16 && n % 4 == 0 && ldo % 4 == 0 && al16(partial) && al16(out) && al16(xpart) && al16(xout)) {
     if (pdl_enabled()) {  // opt-in (common.cuh)
       GCNB_CUDA(launch_pdl(reduce_partials_vec_kernel<true>, dim3((unsigned)ceil_div(total / 4, 8)), dim3(kThreads), 0, st,
-                           total / 4, n / 4, n_parts, reinterpret_cast<const float4*>(partial), out, ldo, m, extra_row));
+                           total / 4, n / 4, n_parts, reinterpret_cast<const float4*>(partial), out, ldo, m,
+                           reinterpret_cast<const double2*>(xpart), xout));
       return GCNB_OK;
     }
     reduce_partials_vec_kernel<false><<<(unsigned)ceil_div(total / 4, 8), kThreads, 0, st>>>(
-        total / 4, n / 4, n_parts, reinterpret_cast<const float4*>(partial), out, ldo, m, extra_row);
+        total / 4, n / 4, n_parts, reinterpret_cast<const float4*>(partial), out, ldo, m,
+        reinterpret_cast<const double2*>(xpart), xout);
     GCNB_LAUNCH_CHECK();
     return GCNB_OK;
   }
-  reduce_partials_kernel<<<(unsigned)ceil_div(total, 32), kThreads, 0, st>>>(total, n, n_parts, partial,
-                                                                            out, ldo, m, extra_row);
+  reduce_partials_kernel<<<(unsigned)ceil_div(total, 32), kThreads, 0, st>>>(total, n, n_parts, partial, out, ldo, m,
+                                                                            xpart, xout);
   GCNB_LAUNCH_CHECK();
   return GCNB_OK;
 }

@@ -133,12 +133,18 @@ int gemm_fp32_launch(int64_t m, int64_t n, int64_t k, const float* a, int64_t a_
   }
   if (k_per_split == 0) k_per_split = BK;
   const int real_splits = (splits > 1) ? (int)ceil_div(k, k_per_split) : 1;
-#define GCNB_GEMM_LAUNCH(BM_, BN_)                                                              \
-  do {                                                                                          \
-    dim3 grid((unsigned)ceil_div(m, BM_), (unsigned)ceil_div(n, BN_), (unsigned)real_splits);   \
-    gemm_fp32_kernel<BM_, BN_><<<grid, kThreads, 0, st>>>((int)m, (int)n, k, a, a_rs, a_cs, b,  \
-                                                          b_rs, b_cs, dst, dst_ld, k_per_split, \
-                                                          split_stride);                        \
+  // N tiles go on grid y, which holds at most 65535: wider products run as several launches of column panels
+#define GCNB_GEMM_LAUNCH(BM_, BN_)                                                                     \
+  do {                                                                                                 \
+    const int64_t panel = 65535ll * BN_;                                                               \
+    for (int64_t n0 = 0; n0 < n; n0 += panel) {                                                        \
+      const int64_t nc = (n - n0 < panel) ? n - n0 : panel;                                            \
+      dim3 grid((unsigned)ceil_div(m, BM_), (unsigned)ceil_div(nc, BN_), (unsigned)real_splits);       \
+      gemm_fp32_kernel<BM_, BN_><<<grid, kThreads, 0, st>>>((int)m, (int)nc, k, a, a_rs, a_cs,         \
+                                                            b + n0 * b_cs, b_rs, b_cs, dst + n0, dst_ld, \
+                                                            k_per_split, split_stride);                \
+      if (n0 + nc < n) GCNB_LAUNCH_CHECK();                                                            \
+    }                                                                                                  \
   } while (0)
   if (m <= 64) {
     if (n <= 16) GCNB_GEMM_LAUNCH(64, 16);

@@ -110,14 +110,16 @@ skinny_rows_kernel(int64_t M, int N, int K, const float* __restrict__ a, int64_t
 // ---------------------------------------------------------------------------------------------- tn
 // C_partial[cta][Mo][N] = sum over this CTA's rows of X[r, 0:Mo]^T Y[r, 0:N];  MMAX = padded Mo, N <= 32.
 // GSUM: a third operand G [R, N] rides along and its column sums (db = colsum(G), the AddBackward0 of
-// pygcn/layers.py:36) land in row Mo of the partial tile -- the layer's backward then needs no colsum kernel when
-// no mask has to be applied to G first (one launch and one 12.8 MB pass less on the CBG shape).
+// pygcn/layers.py:36) land in gpartial[cta][N], in fp64 like every column sum (elementwise.cu) -- the layer's backward
+// then needs no colsum kernel when no mask has to be applied to G first (one launch and one 12.8 MB pass less on the
+// CBG shape).
 // PDL: the programmatic-dependent-launch instantiation (common.cuh); y is the previous kernel's output, so the wait
 // comes first and only the launch latency and the CTA scheduling overlap.
 template <int MMAX, bool GSUM, bool PDL = false>
 __global__ void __launch_bounds__(kThreads)
 skinny_tn_kernel(int64_t R, int Mo, int N, const float* __restrict__ x, int64_t ldx, const float* __restrict__ y,
-                 int64_t ldy, const float* __restrict__ gx, int64_t ldg, float* __restrict__ partial) {
+                 int64_t ldy, const float* __restrict__ gx, int64_t ldg, float* __restrict__ partial,
+                 double* __restrict__ gpartial) {
   if constexpr (PDL) {
     pdl_launch_dependents();
     pdl_wait();
@@ -190,7 +192,8 @@ skinny_tn_kernel(int64_t R, int Mo, int N, const float* __restrict__ x, int64_t 
   cp_async_wait<0>();
   __syncthreads();
   // CTA reduction in a fixed order: warp w adds into the shared tile in turn (w = 0 initialises)
-  float* tile = &xs[0][0][0][0];  // (MMAX + 1) * 32 floats <= the xs array (kWarps*2*8*MMAX floats)
+  float* tile = &xs[0][0][0][0];  // MMAX * 32 floats + 32 doubles <= the xs array (kWarps*2*8*MMAX floats)
+  double* gtile = reinterpret_cast<double*>(tile + MMAX * 32);
   for (int wv = 0; wv < kWarps; ++wv) {
     if (warp == wv) {
 #pragma unroll
@@ -198,16 +201,14 @@ skinny_tn_kernel(int64_t R, int Mo, int N, const float* __restrict__ x, int64_t 
         const float prev = (wv == 0) ? 0.f : tile[k * 32 + lane];
         tile[k * 32 + lane] = prev + acc[k];
       }
-      if constexpr (GSUM) tile[MMAX * 32 + lane] = ((wv == 0) ? 0.f : tile[MMAX * 32 + lane]) + (float)gacc;
+      if constexpr (GSUM) gtile[lane] = ((wv == 0) ? 0.0 : gtile[lane]) + gacc;
     }
     __syncthreads();
   }
-  const int rows_out = GSUM ? Mo + 1 : Mo;  // row Mo of the partial tile = column sums of G
-  float* dst = partial + (int64_t)blockIdx.x * rows_out * N;
-  for (int i = threadIdx.x; i < rows_out * N; i += kThreads) {
-    const int k = i / N;
-    dst[i] = tile[((GSUM && k == Mo) ? MMAX : k) * 32 + (i % N)];
-  }
+  float* dst = partial + (int64_t)blockIdx.x * Mo * N;
+  for (int i = threadIdx.x; i < Mo * N; i += kThreads) dst[i] = tile[(i / N) * 32 + (i % N)];
+  if constexpr (GSUM)
+    if (threadIdx.x < N) gpartial[(int64_t)blockIdx.x * N + threadIdx.x] = gtile[threadIdx.x];
 }
 
 inline bool al16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
@@ -258,8 +259,13 @@ static int skinny_tn_ctas(int64_t r) {
   return (int)(g < 1 ? 1 : g);
 }
 
+// fp32 partial tiles [ctas][m][n], then (256-byte aligned) the fp64 column sums of the fused db [ctas][n]
+static size_t skinny_tn_tile_bytes(int64_t m, int64_t n, int64_t r) {
+  return ((size_t)skinny_tn_ctas(r) * (size_t)m * (size_t)n * sizeof(float) + 255) & ~(size_t)255;
+}
+
 size_t gemm_skinny_tn_workspace_bytes(int64_t m, int64_t n, int64_t r) {
-  return (size_t)skinny_tn_ctas(r) * (size_t)(m + 1) * (size_t)n * sizeof(float);  // (+1: the colsum row)
+  return skinny_tn_tile_bytes(m, n, r) + (size_t)skinny_tn_ctas(r) * (size_t)n * sizeof(double);
 }
 
 // per-device opt-in above the static 48 KB limit (MMAX = 64 with the third operand: 64 KB)
@@ -278,16 +284,16 @@ static int skinny_tn_allow_smem(size_t smem) {
 
 template <int MMAX, bool GSUM>
 static int skinny_tn_launch_t(int ctas, int64_t r, int m, int n, const float* x, int64_t ldx, const float* y, int64_t ldy,
-                              const float* gx, int64_t ldg, float* partial, cudaStream_t st) {
+                              const float* gx, int64_t ldg, float* partial, double* gpartial, cudaStream_t st) {
   const size_t smem = (size_t)kWarps * 2 * kStageRows * (MMAX + 32 + (GSUM ? 32 : 0)) * sizeof(float);
   if (pdl_enabled()) {  // opt-in (common.cuh)
     GCNB_TRY((skinny_tn_allow_smem<MMAX, GSUM, true>(smem)));
     GCNB_CUDA(launch_pdl(skinny_tn_kernel<MMAX, GSUM, true>, dim3((unsigned)ctas), dim3(kThreads), smem, st, r, m, n, x, ldx,
-                         y, ldy, gx, ldg, partial));
+                         y, ldy, gx, ldg, partial, gpartial));
     return GCNB_OK;
   }
   GCNB_TRY((skinny_tn_allow_smem<MMAX, GSUM, false>(smem)));
-  skinny_tn_kernel<MMAX, GSUM><<<ctas, kThreads, smem, st>>>(r, m, n, x, ldx, y, ldy, gx, ldg, partial);
+  skinny_tn_kernel<MMAX, GSUM><<<ctas, kThreads, smem, st>>>(r, m, n, x, ldx, y, ldy, gx, ldg, partial, gpartial);
   GCNB_LAUNCH_CHECK();
   return GCNB_OK;
 }
@@ -298,20 +304,21 @@ int gemm_skinny_tn_launch(int64_t m, int64_t n, int64_t r, const float* x, int64
                           float* db) {
   const int ctas = skinny_tn_ctas(r);
   GCNB_REQUIRE(ws != nullptr && ws_bytes >= gemm_skinny_tn_workspace_bytes(m, n, r), "gemm(skinny tn): workspace too small");
-  GCNB_REQUIRE(gx == nullptr || (db != nullptr && ldg % 4 == 0 && ldg >= n && al16(gx)),
-               "gemm(skinny tn): the fused column sum needs 16-byte aligned rows of G and an output");
+  GCNB_REQUIRE(gx == nullptr || (db != nullptr && ldg % 4 == 0 && ldg >= n && al16(gx) && al16(ws)),
+               "gemm(skinny tn): the fused column sum needs 16-byte aligned rows of G and workspace, and an output");
   float* partial = reinterpret_cast<float*>(ws);
+  double* gpartial = reinterpret_cast<double*>(reinterpret_cast<char*>(ws) + skinny_tn_tile_bytes(m, n, r));
   int status;
 #define GCNB_SKINNY_TN(MMAX_)                                                                                              \
-  status = gx ? (skinny_tn_launch_t<MMAX_, true>(ctas, r, (int)m, (int)n, x, ldx, y, ldy, gx, ldg, partial, st))           \
-              : (skinny_tn_launch_t<MMAX_, false>(ctas, r, (int)m, (int)n, x, ldx, y, ldy, nullptr, 0, partial, st))
+  status = gx ? (skinny_tn_launch_t<MMAX_, true>(ctas, r, (int)m, (int)n, x, ldx, y, ldy, gx, ldg, partial, gpartial, st)) \
+              : (skinny_tn_launch_t<MMAX_, false>(ctas, r, (int)m, (int)n, x, ldx, y, ldy, nullptr, 0, partial, nullptr, st))
   if (m <= 8) GCNB_SKINNY_TN(8);
   else if (m <= 16) GCNB_SKINNY_TN(16);
   else if (m <= 32) GCNB_SKINNY_TN(32);
   else GCNB_SKINNY_TN(64);
 #undef GCNB_SKINNY_TN
   GCNB_TRY(status);
-  return reduce_partials_launch(m, n, ctas, partial, c, ldc, st, gx ? db : nullptr);
+  return reduce_partials_launch(m, n, ctas, partial, c, ldc, st, gx ? gpartial : nullptr, gx ? db : nullptr);
 }
 
 }  // namespace gcnb

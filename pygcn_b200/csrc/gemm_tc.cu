@@ -470,13 +470,13 @@ gemm_tc_tn_tma_kernel(const __grid_constant__ TmaDesc tmap_x, const __grid_const
   tc_fence_after();
   const uint32_t tmem_base = *reinterpret_cast<volatile uint32_t*>(gen + tmem_slot_off);
 
-  const int m0 = blockIdx.y * BM;
-  const int64_t r_begin = (int64_t)blockIdx.x * rows_per_split;
+  const int m0 = blockIdx.x * BM;  // (M tiles on x: y would cap them at 65535, M at 8.4 M)
+  const int64_t r_begin = (int64_t)blockIdx.y * rows_per_split;
   const int64_t r_end = min(R, r_begin + rows_per_split);
   const int nkb = (r_end > r_begin) ? (int)((r_end - r_begin + BKF - 1) / BKF) : 0;
   const int n_chunks = (nkb + kTnDrainBlocks - 1) / kTnDrainBlocks;
   const int ng = npad >> 5;
-  float* cdst = c + (int64_t)blockIdx.x * split_stride;
+  float* cdst = c + (int64_t)blockIdx.y * split_stride;
 
   if (warp == 5) {
     // ===================== TMA producer =====================
@@ -847,7 +847,7 @@ int gemm_tc_tn_launch(int64_t m, int64_t n, int64_t r, const float* x, int64_t l
   const int64_t stride = (t.splits > 1) ? m * n : 0;
   const int vec = (ld % 4 == 0) && aligned16(dst);
   GCNB_TRY(allow_big_smem(reinterpret_cast<const void*>(gemm_tc_tn_tma_kernel), 1));
-  gemm_tc_tn_tma_kernel<<<dim3((unsigned)t.splits, (unsigned)t.m_tiles), kTmaThreads, t.smem, st>>>(
+  gemm_tc_tn_tma_kernel<<<dim3((unsigned)t.m_tiles, (unsigned)t.splits), kTmaThreads, t.smem, st>>>(
       tx, ty, r, (int)m, (int)n, dst, ld, stride, t.rows_per_split, t.npad, tmem_cols_for(2 * t.npad), vec, t.ns);
   GCNB_LAUNCH_CHECK();
   if (t.splits > 1) GCNB_TRY(reduce_partials_launch(m, n, (int)t.splits, dst, c, ldc, st));
