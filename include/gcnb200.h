@@ -57,6 +57,7 @@ int gcnb_check_device(void);
 #define GCNB_BUILD_SELF_LOOPS 2    /* A <- A + I (fp64)                pygcn/utils.py:368 */
 #define GCNB_BUILD_ROW_NORMALIZE 4 /* A <- D^-1 A, fp64, inf -> 0      pygcn/utils.py:390-397 */
 #define GCNB_BUILD_CORA_PIPELINE 7
+#define GCNB_BUILD_KEEP_F64 8      /* also keep the fp64 values (before the cast of utils.py:409): an fp64 handle */
 
 /* Row-length bins of the schedule (deg = stored entries in the row):
  *   0: deg == 0   1: 1..8   2: 9..32   3: 33..1024   4: > 1024 (split across warps)   */
@@ -89,6 +90,17 @@ int gcnb_graph_from_csr(int64_t n_rows, int64_t n_cols, int64_t nnz, const int64
  * policy-generator.py:339): non-zeros are scanned into CSR on the device.  sync. */
 int gcnb_graph_from_dense(int64_t n_rows, int64_t n_cols, const float* d_a, int64_t lda,
                           void* stream, gcnb_graph** out);
+
+/* fp64 handles.  The same builds on double values: same sort, duplicate handling, transpose and schedule; the
+ * handle keeps the fp64 values for the _f64 products below and, as val / t_val, their fp32 rounding (so the fp32
+ * entry points, the exports and gcnb_graph_block work on it as on any handle).  A dense fp64 adjacency is scanned into
+ * CSR: fp64 handles never take the dense route.  d_val / d_a 8-byte aligned.  sync. */
+int gcnb_graph_from_coo_f64(int64_t n_rows, int64_t n_cols, int64_t nnz, const int64_t* d_row,
+                            const int64_t* d_col, const double* d_val, void* stream, gcnb_graph** out);
+int gcnb_graph_from_csr_f64(int64_t n_rows, int64_t n_cols, int64_t nnz, const int64_t* d_crow,
+                            const int64_t* d_col, const double* d_val, void* stream, gcnb_graph** out);
+int gcnb_graph_from_dense_f64(int64_t n_rows, int64_t n_cols, const double* d_a, int64_t lda,
+                              void* stream, gcnb_graph** out);
 
 void gcnb_graph_free(gcnb_graph* g);
 
@@ -144,6 +156,10 @@ int gcnb_graph_block_sources(const gcnb_graph* g, int transpose, int64_t r0, int
  * buffers: d_rowptr int32 [rows+1], d_col int32 [nnz], d_val fp32 [nnz]. */
 int gcnb_graph_export_csr(const gcnb_graph* g, int transpose, int32_t* d_rowptr, int32_t* d_col,
                           float* d_val, void* stream);
+
+/* gcnb_graph_export_csr with the fp64 values; GCNB_E_UNSUPPORTED for a handle that has none. */
+int gcnb_graph_export_csr_f64(const gcnb_graph* g, int transpose, int32_t* d_rowptr, int32_t* d_col,
+                              double* d_val64, void* stream);
 
 /* ------------------------------------------------------------------------------------
  * Hot path kernels
@@ -244,6 +260,41 @@ int gcnb_layer_backward(const gcnb_graph* g, const float* d_x, int64_t ldx, cons
                         float* d_db, float* d_dx, int64_t lddx, void* d_ws, size_t ws_bytes,
                         void* stream);
 size_t gcnb_layer_workspace_bytes(const gcnb_graph* g, int64_t fin, int64_t fout, int precision);
+
+/* ---- fp64 tier: the layer's products, column sums and layer entry points on double operands --------------------
+ * What `model.double()` runs in the reference (torch.mm / torch.spmm on fp64).  Each mirrors the fp32 entry point of
+ * the same name without the `precision` argument: the SpMM reads the handle's fp64 values (handles built by the _f64
+ * constructors or with GCNB_BUILD_KEEP_F64; any other handle is refused with GCNB_E_INVALID), the dense products run on
+ * the fp64 tensor cores (DMMA), the column sums add in fp64 in a fixed order.  Every result is bit-reproducible.
+ * Operands are 8-byte aligned; panels whose rows are 16-byte aligned (even ld, 16-byte aligned base) are gathered with
+ * 16-byte loads, so internal panels use ld2(f) = 2*ceil(f/2).  Workspaces: the matching *_workspace_bytes, 8-byte
+ * aligned. */
+/* gcnb_spmm with the dropout epilogue: out = dropout(relu(A b (+ out) (+ bias))), d_mask NULL or uint8 [rows, ld_mask] */
+int gcnb_spmm_f64(const gcnb_graph* g, int flags, const double* d_b, int64_t ldb, int64_t f, const double* d_bias,
+                  const uint8_t* d_mask, int64_t ld_mask, double mask_scale, double* d_out, int64_t ldo, void* d_ws,
+                  size_t ws_bytes, void* stream);
+size_t gcnb_spmm_f64_workspace_bytes(const gcnb_graph* g, int flags, int64_t f);
+int gcnb_gemm_f64(int64_t m, int64_t n, int64_t k, const double* d_a, int64_t a_rs, int64_t a_cs, const double* d_b,
+                  int64_t b_rs, int64_t b_cs, double* d_c, int64_t ldc, void* d_ws, size_t ws_bytes, void* stream);
+int gcnb_gemm_f64_ex(int64_t m, int64_t n, int64_t k, const double* d_a, int64_t a_rs, int64_t a_cs, const double* d_b,
+                     int64_t b_rs, int64_t b_cs, double* d_c, int64_t ldc, const double* d_bias, int relu, void* d_ws,
+                     size_t ws_bytes, void* stream);
+size_t gcnb_gemm_f64_workspace_bytes(int64_t m, int64_t n, int64_t k);
+/* gcnb_colsum in fp64; d_out may be NULL when d_gm is given (only the masked / staged copy is written) */
+int gcnb_colsum_f64(int64_t n_rows, int64_t f, const double* d_g, int64_t ldg, const double* d_y, int64_t ldy,
+                    double* d_gm, int64_t ldgm, double* d_out, void* d_ws, size_t ws_bytes, void* stream);
+size_t gcnb_colsum_f64_workspace_bytes(int64_t n_rows, int64_t f);
+/* as gcnb_layer_forward / _backward with ld2 in place of ld4: d_support [n_cols, ld2(fout)] (AGG_FIRST: A X
+ * [n_rows, ld2(fin)]), d_gm [n_rows, ld2(fout)] (required with RELU or a dropout mask), d_ds [n_cols, ld2(fout)]
+ * (AGG_FIRST: [n_rows, ld2(fin)], dX only) */
+int gcnb_layer_forward_f64(const gcnb_graph* g, const double* d_x, int64_t ldx, const double* d_w, const double* d_bias,
+                           int64_t fin, int64_t fout, int flags, const uint8_t* d_mask, double mask_scale,
+                           double* d_support, double* d_out, void* d_ws, size_t ws_bytes, void* stream);
+int gcnb_layer_backward_f64(const gcnb_graph* g, const double* d_x, int64_t ldx, const double* d_w, const double* d_g,
+                            int64_t ldg, const double* d_y, int64_t fin, int64_t fout, int flags, const uint8_t* d_mask,
+                            double mask_scale, double* d_gm, double* d_ds, double* d_dw, double* d_db, double* d_dx,
+                            int64_t lddx, void* d_ws, size_t ws_bytes, void* stream);
+size_t gcnb_layer_f64_workspace_bytes(const gcnb_graph* g, int64_t fin, int64_t fout);
 
 /* ---- (ReLU ->) fresh training-mode BatchNorm1d over the layer output (SURVEY.md 8f rank 2) ------------------------
  * Replaces pygcn/models.py:41-45 `GCN.apply_bn` (a NEW nn.BatchNorm1d(F) per call: affine weight 1 / bias 0, batch

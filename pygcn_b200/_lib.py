@@ -17,12 +17,13 @@ c_i64 = ctypes.c_int64
 c_int = ctypes.c_int
 c_vp = ctypes.c_void_p
 c_sz = ctypes.c_size_t
+c_double = ctypes.c_double
 
 NUM_BINS = 5
 BIN_EDGES = (0, 1, 9, 33, 1025)
 
 # flags (mirror include/gcnb200.h)
-BUILD_SYMMETRIZE, BUILD_SELF_LOOPS, BUILD_ROW_NORMALIZE = 1, 2, 4
+BUILD_SYMMETRIZE, BUILD_SELF_LOOPS, BUILD_ROW_NORMALIZE, BUILD_KEEP_F64 = 1, 2, 4, 8
 SPMM_TRANSPOSE, SPMM_RELU, SPMM_ACCUMULATE = 1, 2, 4
 GEMM_FP32, GEMM_TF32X3, GEMM_AUTO = 0, 1, 2
 LAYER_RELU, LAYER_NEED_DX, LAYER_NEED_DW, LAYER_NEED_DB, LAYER_AGG_FIRST = 1, 2, 4, 8, 16
@@ -103,6 +104,24 @@ SIGNATURES = {
     "gcnb_halo_nccl_available": (c_int, []),
     "gcnb_halo_pack": (c_int, [c_vp, c_vp, c_i64, c_i64, c_vp, c_vp]),
     "gcnb_halo_exchange": (c_int, [c_vp, c_vp, c_vp, c_i64, c_vp, c_vp]),
+    # fp64 tier
+    "gcnb_graph_from_coo_f64": (c_int, [c_i64, c_i64, c_i64, c_vp, c_vp, c_vp, c_vp, ctypes.POINTER(c_vp)]),
+    "gcnb_graph_from_csr_f64": (c_int, [c_i64, c_i64, c_i64, c_vp, c_vp, c_vp, c_vp, ctypes.POINTER(c_vp)]),
+    "gcnb_graph_from_dense_f64": (c_int, [c_i64, c_i64, c_vp, c_i64, c_vp, ctypes.POINTER(c_vp)]),
+    "gcnb_graph_export_csr_f64": (c_int, [c_vp, c_int, c_vp, c_vp, c_vp, c_vp]),
+    "gcnb_spmm_f64": (c_int, [c_vp, c_int, c_vp, c_i64, c_i64, c_vp, c_vp, c_i64, c_double, c_vp, c_i64, c_vp, c_sz, c_vp]),
+    "gcnb_spmm_f64_workspace_bytes": (c_sz, [c_vp, c_int, c_i64]),
+    "gcnb_gemm_f64": (c_int, [c_i64, c_i64, c_i64, c_vp, c_i64, c_i64, c_vp, c_i64, c_i64, c_vp, c_i64, c_vp, c_sz, c_vp]),
+    "gcnb_gemm_f64_ex": (c_int, [c_i64, c_i64, c_i64, c_vp, c_i64, c_i64, c_vp, c_i64, c_i64, c_vp, c_i64, c_vp, c_int,
+                                 c_vp, c_sz, c_vp]),
+    "gcnb_gemm_f64_workspace_bytes": (c_sz, [c_i64, c_i64, c_i64]),
+    "gcnb_colsum_f64": (c_int, [c_i64, c_i64, c_vp, c_i64, c_vp, c_i64, c_vp, c_i64, c_vp, c_vp, c_sz, c_vp]),
+    "gcnb_colsum_f64_workspace_bytes": (c_sz, [c_i64, c_i64]),
+    "gcnb_layer_forward_f64": (c_int, [c_vp, c_vp, c_i64, c_vp, c_vp, c_i64, c_i64, c_int, c_vp, c_double, c_vp, c_vp,
+                                       c_vp, c_sz, c_vp]),
+    "gcnb_layer_backward_f64": (c_int, [c_vp, c_vp, c_i64, c_vp, c_vp, c_i64, c_vp, c_i64, c_i64, c_int, c_vp, c_double,
+                                        c_vp, c_vp, c_vp, c_vp, c_vp, c_i64, c_vp, c_sz, c_vp]),
+    "gcnb_layer_f64_workspace_bytes": (c_sz, [c_vp, c_i64, c_i64]),
 }
 
 _lock = threading.Lock()

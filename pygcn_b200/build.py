@@ -20,7 +20,7 @@ CSRC = os.path.join(HERE, "csrc")
 LIBDIR = os.path.join(HERE, "lib")
 LIB = os.path.join(LIBDIR, "libgcnb200.so")
 
-SOURCES = ["api.cu", "spmm.cu", "spmm_stream.cu", "gemm_simt.cu", "gemm_skinny.cu", "gemm_tc.cu", "elementwise.cu", "graph_build.cu", "peer.cu", "batchnorm.cu", "dist.cu"]
+SOURCES = ["api.cu", "spmm.cu", "spmm_stream.cu", "gemm_simt.cu", "gemm_skinny.cu", "gemm_tc.cu", "elementwise.cu", "graph_build.cu", "peer.cu", "batchnorm.cu", "dist.cu", "spmm_f64.cu", "gemm_f64.cu"]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",

@@ -458,3 +458,202 @@ extern "C" int gcnb_layer_backward(const gcnb_graph* g, const float* d_x, int64_
   }
   return GCNB_OK;
 }
+
+// ------------------------------------------------------------------------ fp64 tier
+
+namespace gcnb {
+namespace {
+
+inline int64_t ld2(int64_t f) { return ceil_div(f, 2) * 2; }
+
+int require_f64(const gcnb_graph* g, bool transpose, const char* what) {
+  GCNB_REQUIRE(g != nullptr, "%s: null graph", what);
+  GCNB_REQUIRE(g->val64 != nullptr,
+               "%s: the graph handle has no fp64 values (build it with a gcnb_graph_from_*_f64 constructor or "
+               "GCNB_BUILD_KEEP_F64)", what);
+  GCNB_REQUIRE(!transpose || (g->has_transpose && g->t_val64 != nullptr), "%s: this handle has no transpose", what);
+  return GCNB_OK;
+}
+
+int spmm_f64_graph(const gcnb_graph* g, bool transpose, const double* b, int64_t ldb, int64_t f, const Epilogue64& ep,
+                   double* out, int64_t ldo, void* ws, size_t ws_bytes, cudaStream_t st) {
+  return spmm_f64_launch(transpose ? g->bwd : g->fwd, transpose ? g->t_val64 : g->val64, b, ldb, f, ep, out, ldo, ws,
+                         ws_bytes, st);
+}
+
+Epilogue64 make_epilogue64(const double* bias, bool relu, bool accumulate, const uint8_t* mask, int64_t ld_mask,
+                           double scale) {
+  Epilogue64 ep;
+  ep.bias = bias;
+  ep.relu = relu ? 1 : 0;
+  ep.accumulate = accumulate ? 1 : 0;
+  ep.mask = mask;
+  ep.ld_mask = ld_mask;
+  ep.mask_scale = scale;
+  return ep;
+}
+
+struct LayerF64Ws {
+  size_t s, c, d;
+};
+
+LayerF64Ws layer_f64_regions(const gcnb_graph* g, int64_t fin, int64_t fout) {
+  LayerF64Ws r{0, 0, 0};
+  for (int64_t w : {fout, fin})
+    for (const CsrView* v : {&g->fwd, &g->bwd}) {
+      const size_t b = spmm_f64_workspace_bytes(*v, w);
+      if (b > r.s) r.s = b;
+    }
+  r.c = colsum_f64_workspace_bytes(g->n_rows, fout);
+  const size_t d[6] = {gemm_f64_workspace_bytes(g->n_cols, fout, fin),   // X W
+                       gemm_f64_workspace_bytes(fin, fout, g->n_cols),   // X^T dS
+                       gemm_f64_workspace_bytes(g->n_cols, fin, fout),   // dS W^T
+                       gemm_f64_workspace_bytes(g->n_rows, fout, fin),   // (A X) W
+                       gemm_f64_workspace_bytes(g->n_rows, fin, fout),   // G W^T
+                       gemm_f64_workspace_bytes(fin, fout, g->n_rows)};  // (A X)^T G
+  for (size_t v : d)
+    if (v > r.d) r.d = v;
+  r.s = align256(r.s);
+  r.c = align256(r.c);
+  r.d = align256(r.d);
+  return r;
+}
+
+}  // namespace
+}  // namespace gcnb
+
+extern "C" int gcnb_spmm_f64(const gcnb_graph* g, int flags, const double* d_b, int64_t ldb, int64_t f,
+                             const double* d_bias, const uint8_t* d_mask, int64_t ld_mask, double mask_scale,
+                             double* d_out, int64_t ldo, void* d_ws, size_t ws_bytes, void* stream) {
+  const bool transpose = (flags & GCNB_SPMM_TRANSPOSE) != 0;
+  GCNB_TRY(require_f64(g, transpose, "spmm_f64"));
+  GCNB_REQUIRE((flags & ~(GCNB_SPMM_TRANSPOSE | GCNB_SPMM_RELU | GCNB_SPMM_ACCUMULATE)) == 0, "spmm_f64: unknown flags");
+  return spmm_f64_graph(g, transpose, d_b, ldb, f,
+                        make_epilogue64(d_bias, (flags & GCNB_SPMM_RELU) != 0, (flags & GCNB_SPMM_ACCUMULATE) != 0, d_mask,
+                                        ld_mask, mask_scale),
+                        d_out, ldo, d_ws, ws_bytes, (cudaStream_t)stream);
+}
+
+extern "C" size_t gcnb_spmm_f64_workspace_bytes(const gcnb_graph* g, int flags, int64_t f) {
+  if (!g) return 0;
+  return spmm_f64_workspace_bytes((flags & GCNB_SPMM_TRANSPOSE) ? g->bwd : g->fwd, f);
+}
+
+extern "C" int gcnb_gemm_f64(int64_t m, int64_t n, int64_t k, const double* d_a, int64_t a_rs, int64_t a_cs,
+                             const double* d_b, int64_t b_rs, int64_t b_cs, double* d_c, int64_t ldc, void* d_ws,
+                             size_t ws_bytes, void* stream) {
+  return gemm_f64_launch(m, n, k, d_a, a_rs, a_cs, d_b, b_rs, b_cs, d_c, ldc, Epilogue64(), d_ws, ws_bytes,
+                         (cudaStream_t)stream);
+}
+
+extern "C" int gcnb_gemm_f64_ex(int64_t m, int64_t n, int64_t k, const double* d_a, int64_t a_rs, int64_t a_cs,
+                                const double* d_b, int64_t b_rs, int64_t b_cs, double* d_c, int64_t ldc,
+                                const double* d_bias, int relu, void* d_ws, size_t ws_bytes, void* stream) {
+  return gemm_f64_launch(m, n, k, d_a, a_rs, a_cs, d_b, b_rs, b_cs, d_c, ldc,
+                         make_epilogue64(d_bias, relu != 0, false, nullptr, 0, 1.0), d_ws, ws_bytes, (cudaStream_t)stream);
+}
+
+extern "C" size_t gcnb_gemm_f64_workspace_bytes(int64_t m, int64_t n, int64_t k) { return gemm_f64_workspace_bytes(m, n, k); }
+
+extern "C" int gcnb_colsum_f64(int64_t n_rows, int64_t f, const double* d_g, int64_t ldg, const double* d_y,
+                               int64_t ldy, double* d_gm, int64_t ldgm, double* d_out, void* d_ws, size_t ws_bytes,
+                               void* stream) {
+  return colsum_f64_launch(n_rows, f, d_g, ldg, d_y, ldy, d_gm, ldgm, d_out, d_ws, ws_bytes, (cudaStream_t)stream);
+}
+
+extern "C" size_t gcnb_colsum_f64_workspace_bytes(int64_t n_rows, int64_t f) { return colsum_f64_workspace_bytes(n_rows, f); }
+
+extern "C" size_t gcnb_layer_f64_workspace_bytes(const gcnb_graph* g, int64_t fin, int64_t fout) {
+  if (!g) return 0;
+  const LayerF64Ws r = layer_f64_regions(g, fin, fout);
+  return r.s + r.c + r.d + 256;
+}
+
+extern "C" int gcnb_layer_forward_f64(const gcnb_graph* g, const double* d_x, int64_t ldx, const double* d_w,
+                                      const double* d_bias, int64_t fin, int64_t fout, int flags, const uint8_t* d_mask,
+                                      double mask_scale, double* d_support, double* d_out, void* d_ws, size_t ws_bytes,
+                                      void* stream) {
+  GCNB_TRY(require_f64(g, false, "layer_forward_f64"));
+  GCNB_REQUIRE(fin > 0 && fout > 0 && fin < (1ll << 31) && fout < (1ll << 31), "layer_forward_f64: bad feature sizes %lld -> %lld",
+               (long long)fin, (long long)fout);
+  GCNB_REQUIRE(ldx >= fin, "layer_forward_f64: ldx < in_features");
+  GCNB_REQUIRE(d_w != nullptr && d_support != nullptr && d_out != nullptr && (d_x != nullptr || g->n_cols == 0),
+               "layer_forward_f64: null operand");
+  const size_t need = gcnb_layer_f64_workspace_bytes(g, fin, fout);
+  GCNB_REQUIRE(d_ws != nullptr && ws_bytes >= need, "layer_forward_f64: workspace too small (%zu < %zu)", ws_bytes, need);
+  const LayerF64Ws r = layer_f64_regions(g, fin, fout);
+  cudaStream_t st = (cudaStream_t)stream;
+  char* ws = reinterpret_cast<char*>(d_ws);
+  const Epilogue64 ep = make_epilogue64(d_bias, (flags & GCNB_LAYER_RELU) != 0, false, d_mask, fout, mask_scale);
+  if (flags & GCNB_LAYER_AGG_FIRST) {  // out = (A X) W + bias; d_support receives A X [n_rows, ld2(fin)] for backward
+    const int64_t ldax = ld2(fin);
+    GCNB_TRY(spmm_f64_graph(g, false, d_x, ldx, fin, Epilogue64(), d_support, ldax, ws, r.s, st));
+    return gemm_f64_launch(g->n_rows, fout, fin, d_support, ldax, 1, d_w, fout, 1, d_out, fout, ep, ws + r.s + r.c, r.d, st);
+  }
+  const int64_t lds = ld2(fout);  // support = X W ; out = A support (+ bias) (relu) (dropout)
+  GCNB_TRY(gemm_f64_launch(g->n_cols, fout, fin, d_x, ldx, 1, d_w, fout, 1, d_support, lds, Epilogue64(), ws + r.s + r.c,
+                           r.d, st));
+  return spmm_f64_graph(g, false, d_support, lds, fout, ep, d_out, fout, ws, r.s, st);
+}
+
+extern "C" int gcnb_layer_backward_f64(const gcnb_graph* g, const double* d_x, int64_t ldx, const double* d_w,
+                                       const double* d_g, int64_t ldg, const double* d_y, int64_t fin, int64_t fout,
+                                       int flags, const uint8_t* d_mask, double mask_scale, double* d_gm, double* d_ds,
+                                       double* d_dw, double* d_db, double* d_dx, int64_t lddx, void* d_ws,
+                                       size_t ws_bytes, void* stream) {
+  GCNB_TRY(require_f64(g, true, "layer_backward_f64"));
+  GCNB_REQUIRE(fin > 0 && fout > 0 && fin < (1ll << 31) && fout < (1ll << 31), "layer_backward_f64: bad feature sizes");
+  GCNB_REQUIRE(ldg >= fout && (d_g != nullptr || g->n_rows == 0), "layer_backward_f64: null G or ldg < out_features");
+  const bool relu = (flags & GCNB_LAYER_RELU) != 0;
+  const bool need_dx = (flags & GCNB_LAYER_NEED_DX) != 0;
+  const bool need_dw = (flags & GCNB_LAYER_NEED_DW) != 0;
+  const bool need_db = (flags & GCNB_LAYER_NEED_DB) != 0;
+  const bool agg_first = (flags & GCNB_LAYER_AGG_FIRST) != 0;
+  const bool masked = relu || d_mask != nullptr;
+  GCNB_REQUIRE(!relu || d_y != nullptr, "layer_backward_f64: relu needs y");
+  GCNB_REQUIRE(!masked || d_gm != nullptr, "layer_backward_f64: relu / dropout mask needs gm");
+  GCNB_REQUIRE(!need_db || d_db != nullptr, "layer_backward_f64: db requested but null");
+  GCNB_REQUIRE(!need_dw || d_dw != nullptr, "layer_backward_f64: dW requested but null");
+  GCNB_REQUIRE(!need_dx || (d_dx != nullptr && lddx >= fin), "layer_backward_f64: dX requested but null / lddx < in_features");
+  GCNB_REQUIRE(!(need_dw || need_dx) || ((d_x != nullptr || !need_dw) && ldx >= fin && d_w != nullptr),
+               "layer_backward_f64: null X / W or ldx < in_features");
+  GCNB_REQUIRE(!(agg_first ? need_dx : (need_dx || need_dw)) || d_ds != nullptr, "layer_backward_f64: null ds");
+  const size_t need = gcnb_layer_f64_workspace_bytes(g, fin, fout);
+  GCNB_REQUIRE(d_ws != nullptr && ws_bytes >= need, "layer_backward_f64: workspace too small (%zu < %zu)", ws_bytes, need);
+  const LayerF64Ws r = layer_f64_regions(g, fin, fout);
+  cudaStream_t st = (cudaStream_t)stream;
+  char* ws = reinterpret_cast<char*>(d_ws);
+  void* ws_spmm = ws;
+  void* ws_col = ws + r.s;
+  void* ws_gemm = ws + r.s + r.c;
+  // db = colsum(G); with ReLU / dropout the masked gradient is staged in gm [n_rows, ld2(fout)] and read from there on
+  const double* gsrc = d_g;
+  int64_t gld = ldg;
+  if (masked || need_db) {
+    GCNB_TRY(colsum_f64_launch(g->n_rows, fout, d_g, ldg, relu ? d_y : nullptr, fout, masked ? d_gm : nullptr, ld2(fout),
+                               need_db ? d_db : nullptr,
+                               ws_col, r.c, st, d_mask, fout, mask_scale));
+    if (masked) {
+      gsrc = d_gm;
+      gld = ld2(fout);
+    }
+  }
+  if (!need_dw && !need_dx) return GCNB_OK;
+  if (agg_first) {  // d_x = A X [n_rows, ld2(fin)] from the forward: dW = (A X)^T G ; dX = A^T (G W^T)
+    if (need_dw)
+      GCNB_TRY(gemm_f64_launch(fin, fout, g->n_rows, d_x, 1, ldx, gsrc, gld, 1, d_dw, fout, Epilogue64(), ws_gemm, r.d, st));
+    if (need_dx) {
+      const int64_t ldt = ld2(fin);
+      GCNB_TRY(gemm_f64_launch(g->n_rows, fin, fout, gsrc, gld, 1, d_w, 1, fout, d_ds, ldt, Epilogue64(), ws_gemm, r.d, st));
+      GCNB_TRY(spmm_f64_graph(g, true, d_ds, ldt, fin, Epilogue64(), d_dx, lddx, ws_spmm, r.s, st));
+    }
+    return GCNB_OK;
+  }
+  const int64_t lds = ld2(fout);  // dS = A^T G ; dW = X^T dS ; dX = dS W^T
+  GCNB_TRY(spmm_f64_graph(g, true, gsrc, gld, fout, Epilogue64(), d_ds, lds, ws_spmm, r.s, st));
+  if (need_dw)
+    GCNB_TRY(gemm_f64_launch(fin, fout, g->n_cols, d_x, 1, ldx, d_ds, lds, 1, d_dw, fout, Epilogue64(), ws_gemm, r.d, st));
+  if (need_dx)
+    GCNB_TRY(gemm_f64_launch(g->n_cols, fin, fout, d_ds, lds, 1, d_w, 1, fout, d_dx, lddx, Epilogue64(), ws_gemm, r.d, st));
+  return GCNB_OK;
+}

@@ -195,6 +195,30 @@ int bias_act_launch(int64_t n_rows, int64_t f, float* out, int64_t ldo, const Ep
 int reduce_partials_launch(int64_t m, int64_t n, int n_parts, const float* partial, float* out,
                            int64_t ldo, cudaStream_t stream, const double* xpart = nullptr, float* xout = nullptr);
 
+// ---- fp64 tier (spmm_f64.cu, gemm_f64.cu): the same products and epilogue on fp64 operands, over the fp64 values a
+// handle keeps when it was built from fp64 data (gcnb_graph::val64 / t_val64)
+struct Epilogue64 {
+  const double* bias = nullptr;   // [f] or null
+  int relu = 0;
+  int accumulate = 0;             // add the previous contents of out first
+  const uint8_t* mask = nullptr;  // [n_rows, ld_mask] keep-mask (0 / non-zero) or null
+  int64_t ld_mask = 0;
+  double mask_scale = 1.0;
+};
+
+// val: the view's fp64 values (g->val64 for g->fwd, g->t_val64 for g->bwd)
+int spmm_f64_launch(const CsrView& a, const double* val, const double* b, int64_t ldb, int64_t f,
+                    const Epilogue64& ep, double* out, int64_t ldo, void* ws, size_t ws_bytes, cudaStream_t stream);
+size_t spmm_f64_workspace_bytes(const CsrView& a, int64_t f);
+int gemm_f64_launch(int64_t m, int64_t n, int64_t k, const double* a, int64_t a_rs, int64_t a_cs, const double* b,
+                    int64_t b_rs, int64_t b_cs, double* c, int64_t ldc, const Epilogue64& ep, void* ws, size_t ws_bytes,
+                    cudaStream_t stream);
+size_t gemm_f64_workspace_bytes(int64_t m, int64_t n, int64_t k);
+int colsum_f64_launch(int64_t n_rows, int64_t f, const double* g, int64_t ldg, const double* y, int64_t ldy, double* gm,
+                      int64_t ldgm, double* out, void* ws, size_t ws_bytes, cudaStream_t stream,
+                      const uint8_t* mask = nullptr, int64_t ld_mask = 0, double mask_scale = 1.0);
+size_t colsum_f64_workspace_bytes(int64_t n_rows, int64_t f);
+
 }  // namespace gcnb
 
 struct gcnb_graph {
@@ -223,4 +247,8 @@ struct gcnb_graph {
   uint32_t* t_stream_items = nullptr;
   gcnb::CsrView fwd, bwd;
   int64_t device_bytes = 0;
+  // fp64 values of the CSR and of the CSR of A^T, in the order of val / t_val (whose entries are their fp32 rounding);
+  // only on handles built from fp64 data (gcnb_graph_from_*_f64, GCNB_BUILD_KEEP_F64), null otherwise
+  double* val64 = nullptr;
+  double* t_val64 = nullptr;
 };

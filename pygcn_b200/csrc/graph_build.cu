@@ -414,6 +414,87 @@ __global__ void export_coo_kernel(int64_t nnz, int64_t n_rows, const int32_t* __
   values[e] = val[e];
 }
 
+// ---- fp64 handles: the same pipeline carries val64 beside val, gathered with the same permutations; val = fp32(val64)
+__global__ void gather_coo_f64_kernel(int64_t nnz, const int32_t* __restrict__ perm, const uint64_t* __restrict__ sorted_key,
+                                      const double* __restrict__ val_in, int32_t* __restrict__ row32,
+                                      int32_t* __restrict__ col32, double* __restrict__ val64, float* __restrict__ val) {
+  const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (e >= nnz) return;
+  const uint64_t k = sorted_key[e];
+  row32[e] = (int32_t)(k >> 32);
+  col32[e] = (int32_t)(k & 0xffffffffu);
+  const double v = val_in[perm[e]];
+  val64[e] = v;
+  val[e] = (float)v;
+}
+
+// dst[i] = src[perm[i]] (the transpose's values)
+__global__ void permute_f64_kernel(int64_t nnz, const int32_t* __restrict__ perm, const double* __restrict__ src,
+                                   double* __restrict__ dst) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < nnz) dst[i] = src[perm[i]];
+}
+
+__global__ void round_f64_kernel(int64_t nnz, const double* __restrict__ val64, float* __restrict__ val) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < nnz) val[i] = (float)val64[i];
+}
+
+__global__ void dense_count_f64_kernel(int64_t n_rows, int64_t n_cols, const double* __restrict__ a, int64_t lda,
+                                       int32_t* __restrict__ counts) {
+  const int64_t row = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const int lane = threadIdx.x & 31;
+  if (row >= n_rows) return;
+  int cnt = 0;
+  for (int64_t c0 = 0; c0 < n_cols; c0 += 32) {
+    const int64_t c = c0 + lane;
+    cnt += __popc(__ballot_sync(0xffffffffu, (c < n_cols) && (a[row * lda + c] != 0.0)));
+  }
+  if (lane == 0) counts[row] = cnt;
+}
+
+__global__ void dense_fill_f64_kernel(int64_t n_rows, int64_t n_cols, const double* __restrict__ a, int64_t lda,
+                                      const int32_t* __restrict__ rowptr, int32_t* __restrict__ col,
+                                      double* __restrict__ val64, float* __restrict__ val) {
+  const int64_t row = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const int lane = threadIdx.x & 31;
+  if (row >= n_rows) return;
+  int out = rowptr[row];
+  for (int64_t c0 = 0; c0 < n_cols; c0 += 32) {
+    const int64_t c = c0 + lane;
+    const double v = (c < n_cols) ? a[row * lda + c] : 0.0;
+    const bool nz = (v != 0.0);
+    const unsigned m = __ballot_sync(0xffffffffu, nz);
+    if (nz) {
+      const int off = __popc(m & ((1u << lane) - 1u));
+      col[out + off] = (int32_t)c;
+      val64[out + off] = v;
+      val[out + off] = (float)v;
+    }
+    out += __popc(m);
+  }
+}
+
+// normalize_rows_kernel that also keeps the fp64 values r_inv * value (utils.py:397, before the cast of utils.py:409)
+__global__ void normalize_rows_keep_f64_kernel(int64_t n, const int32_t* __restrict__ rowptr, double* __restrict__ val64,
+                                               int normalize, float* __restrict__ val) {
+  const int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (r >= n) return;
+  const int s = rowptr[r], e = rowptr[r + 1];
+  double r_inv = 1.0;
+  if (normalize) {
+    double sum = 0.0;
+    for (int i = s; i < e; ++i) sum += val64[i];
+    r_inv = 1.0 / sum;
+    if (isinf(r_inv)) r_inv = 0.0;
+  }
+  for (int i = s; i < e; ++i) {
+    const double v = normalize ? r_inv * val64[i] : val64[i];
+    val64[i] = v;
+    val[i] = (float)v;
+  }
+}
+
 int bits_for(uint64_t max_value) {
   int b = 1;
   while (b < 64 && (max_value >> b) != 0) ++b;
@@ -622,6 +703,13 @@ int finalize(gcnb_graph* g, const int32_t* rows, cudaStream_t st, bool with_tran
                                                             g->t_col, g->t_val);
     GCNB_LAUNCH_CHECK();
   }
+  if (g->val64) {
+    GCNB_TRY(graph_alloc(g, &g->t_val64, nnz));
+    if (nnz > 0) {
+      permute_f64_kernel<<<blocks_for(nnz), kT, 0, st>>>(nnz, perm_out.as<int32_t>(), g->val64, g->t_val64);
+      GCNB_LAUNCH_CHECK();
+    }
+  }
   rowptr_from_sorted_kernel<<<blocks_for(g->n_cols + 1), kT, 0, st>>>(key_out.as<int32_t>(), nnz,
                                                                       g->n_cols, g->t_rowptr);
   GCNB_LAUNCH_CHECK();
@@ -686,7 +774,9 @@ int read_flags(DevBuf& flags, int* h, int count, cudaStream_t st) {
   return GCNB_OK;
 }
 
-int from_coo_impl(gcnb_graph* g, const int64_t* row, const int64_t* col, const float* val, cudaStream_t st) {
+// f64: an fp64 handle, values from val64 (val unused)
+int from_coo_impl(gcnb_graph* g, const int64_t* row, const int64_t* col, const float* val, cudaStream_t st,
+                  bool f64 = false, const double* val64 = nullptr) {
   const int64_t nnz = g->nnz;
   DevBuf rows32, key, flags;
   GCNB_TRY(rows32.alloc((size_t)nnz * 4));
@@ -696,9 +786,10 @@ int from_coo_impl(gcnb_graph* g, const int64_t* row, const int64_t* col, const f
   GCNB_TRY(graph_alloc(g, &g->rowptr, g->n_rows + 1));
   GCNB_TRY(graph_alloc(g, &g->col, nnz));
   GCNB_TRY(graph_alloc(g, &g->val, nnz));
+  if (f64) GCNB_TRY(graph_alloc(g, &g->val64, nnz));
   int hf[2] = {0, 0};
   if (nnz > 0) {
-    GCNB_REQUIRE(row && col && val, "graph_from_coo: null input");
+    GCNB_REQUIRE(row && col && (f64 ? val64 != nullptr : val != nullptr), "graph_from_coo: null input");
     coo_convert_kernel<<<blocks_for(nnz), kT, 0, st>>>(nnz, g->n_rows, g->n_cols, row, col,
                                                        rows32.as<int32_t>(), g->col, key.as<uint64_t>(),
                                                        flags.as<int>());
@@ -721,10 +812,18 @@ int from_coo_impl(gcnb_graph* g, const int64_t* row, const int64_t* col, const f
       GCNB_CUDA(cub::DeviceRadixSort::SortPairs(temp.p, tb, key.as<uint64_t>(), key_out.as<uint64_t>(),
                                                 perm_in.as<int32_t>(), perm_out.as<int32_t>(), nnz, 0,
                                                 end_bit, st));
-      gather_coo_kernel<<<blocks_for(nnz), kT, 0, st>>>(nnz, perm_out.as<int32_t>(), key_out.as<uint64_t>(),
-                                                        val, rows32.as<int32_t>(), g->col, g->val);
+      if (f64)
+        gather_coo_f64_kernel<<<blocks_for(nnz), kT, 0, st>>>(nnz, perm_out.as<int32_t>(), key_out.as<uint64_t>(), val64,
+                                                              rows32.as<int32_t>(), g->col, g->val64, g->val);
+      else
+        gather_coo_kernel<<<blocks_for(nnz), kT, 0, st>>>(nnz, perm_out.as<int32_t>(), key_out.as<uint64_t>(),
+                                                          val, rows32.as<int32_t>(), g->col, g->val);
       GCNB_LAUNCH_CHECK();
       GCNB_CUDA(cudaStreamSynchronize(st));
+    } else if (f64) {
+      GCNB_CUDA(cudaMemcpyAsync(g->val64, val64, (size_t)nnz * 8, cudaMemcpyDeviceToDevice, st));
+      round_f64_kernel<<<blocks_for(nnz), kT, 0, st>>>(nnz, g->val64, g->val);
+      GCNB_LAUNCH_CHECK();
     } else {
       GCNB_CUDA(cudaMemcpyAsync(g->val, val, (size_t)nnz * 4, cudaMemcpyDeviceToDevice, st));
     }
@@ -735,9 +834,10 @@ int from_coo_impl(gcnb_graph* g, const int64_t* row, const int64_t* col, const f
   return finalize(g, rows32.as<int32_t>(), st);
 }
 
-int from_csr_impl(gcnb_graph* g, const int64_t* crow, const int64_t* col, const float* val, cudaStream_t st) {
+int from_csr_impl(gcnb_graph* g, const int64_t* crow, const int64_t* col, const float* val, cudaStream_t st,
+                  bool f64 = false, const double* val64 = nullptr) {
   const int64_t nnz = g->nnz;
-  GCNB_REQUIRE(crow != nullptr && (nnz == 0 || (col && val)), "graph_from_csr: null input");
+  GCNB_REQUIRE(crow != nullptr && (nnz == 0 || (col && (f64 ? val64 != nullptr : val != nullptr))), "graph_from_csr: null input");
   DevBuf rows32, flags;
   GCNB_TRY(rows32.alloc((size_t)nnz * 4));
   GCNB_TRY(flags.alloc(2 * sizeof(int)));
@@ -745,6 +845,7 @@ int from_csr_impl(gcnb_graph* g, const int64_t* crow, const int64_t* col, const 
   GCNB_TRY(graph_alloc(g, &g->rowptr, g->n_rows + 1));
   GCNB_TRY(graph_alloc(g, &g->col, nnz));
   GCNB_TRY(graph_alloc(g, &g->val, nnz));
+  if (f64) GCNB_TRY(graph_alloc(g, &g->val64, nnz));
   const int64_t span = (g->n_rows + 1 > nnz) ? g->n_rows + 1 : nnz;
   csr_convert_kernel<<<blocks_for(span), kT, 0, st>>>(g->n_rows, g->n_cols, nnz, crow, col, g->rowptr,
                                                       g->col, flags.as<int>());
@@ -753,7 +854,13 @@ int from_csr_impl(gcnb_graph* g, const int64_t* crow, const int64_t* col, const 
   GCNB_TRY(read_flags(flags, hf, 2, st));
   GCNB_REQUIRE(hf[0] == 0, "graph_from_csr: malformed crow_indices / col_indices");
   if (nnz > 0) {
-    GCNB_CUDA(cudaMemcpyAsync(g->val, val, (size_t)nnz * 4, cudaMemcpyDeviceToDevice, st));
+    if (f64) {
+      GCNB_CUDA(cudaMemcpyAsync(g->val64, val64, (size_t)nnz * 8, cudaMemcpyDeviceToDevice, st));
+      round_f64_kernel<<<blocks_for(nnz), kT, 0, st>>>(nnz, g->val64, g->val);
+      GCNB_LAUNCH_CHECK();
+    } else {
+      GCNB_CUDA(cudaMemcpyAsync(g->val, val, (size_t)nnz * 4, cudaMemcpyDeviceToDevice, st));
+    }
     expand_rows_kernel<<<blocks_for(nnz), kT, 0, st>>>(g->rowptr, g->n_rows, nnz, rows32.as<int32_t>());
     GCNB_LAUNCH_CHECK();
   }
@@ -822,6 +929,51 @@ int from_dense_impl(gcnb_graph** out, int64_t n_rows, int64_t n_cols, const floa
     GCNB_CUDA(cudaStreamSynchronize(st));
   }
   return GCNB_OK;
+}
+
+// fp64 dense adjacency: scanned into CSR (an fp64 handle never takes the dense route)
+int from_dense_f64_impl(gcnb_graph** out, int64_t n_rows, int64_t n_cols, const double* a, int64_t lda, cudaStream_t st) {
+  GCNB_REQUIRE(a != nullptr || n_rows * n_cols == 0, "graph_from_dense_f64: null input");
+  GCNB_REQUIRE(lda >= n_cols, "graph_from_dense_f64: lda < n_cols");
+  GCNB_REQUIRE((reinterpret_cast<uintptr_t>(a) & 7u) == 0, "graph_from_dense_f64: input not 8-byte aligned");
+  DevBuf counts, rowptr, temp, total;
+  GCNB_TRY(counts.alloc((size_t)(n_rows + 1) * 4));
+  GCNB_TRY(rowptr.alloc((size_t)(n_rows + 1) * 4));
+  GCNB_TRY(total.alloc(8));
+  GCNB_CUDA(cudaMemsetAsync(counts.p, 0, (size_t)(n_rows + 1) * 4, st));
+  GCNB_CUDA(cudaMemsetAsync(total.p, 0, 8, st));
+  if (n_rows > 0) {
+    dense_count_f64_kernel<<<blocks_for(n_rows * 32), kT, 0, st>>>(n_rows, n_cols, a, lda, counts.as<int32_t>());
+    GCNB_LAUNCH_CHECK();
+    sum_i32_kernel<<<blocks_for(n_rows), kT, 0, st>>>(counts.as<int32_t>(), n_rows, total.as<unsigned long long>());
+    GCNB_LAUNCH_CHECK();
+  }
+  int64_t nnz = 0;
+  GCNB_CUDA(cudaMemcpyAsync(&nnz, total.p, 8, cudaMemcpyDeviceToHost, st));
+  GCNB_CUDA(cudaStreamSynchronize(st));
+  GCNB_TRY(check_dims(n_rows, n_cols, nnz));
+  size_t tb = 0;
+  GCNB_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, tb, counts.as<int32_t>(), rowptr.as<int32_t>(), (int)(n_rows + 1), st));
+  GCNB_TRY(temp.alloc(tb));
+  GCNB_CUDA(cub::DeviceScan::ExclusiveSum(temp.p, tb, counts.as<int32_t>(), rowptr.as<int32_t>(), (int)(n_rows + 1), st));
+  gcnb_graph* g = new_graph(n_rows, n_cols, nnz);
+  GCNB_REQUIRE(g != nullptr, "graph: host allocation failed");
+  *out = g;
+  DevBuf rows32;
+  GCNB_TRY(rows32.alloc((size_t)nnz * 4));
+  GCNB_TRY(graph_alloc(g, &g->rowptr, n_rows + 1));
+  GCNB_TRY(graph_alloc(g, &g->col, nnz));
+  GCNB_TRY(graph_alloc(g, &g->val, nnz));
+  GCNB_TRY(graph_alloc(g, &g->val64, nnz));
+  GCNB_CUDA(cudaMemcpyAsync(g->rowptr, rowptr.p, (size_t)(n_rows + 1) * 4, cudaMemcpyDeviceToDevice, st));
+  if (n_rows > 0 && nnz > 0) {
+    dense_fill_f64_kernel<<<blocks_for(n_rows * 32), kT, 0, st>>>(n_rows, n_cols, a, lda, g->rowptr, g->col, g->val64,
+                                                                  g->val);
+    GCNB_LAUNCH_CHECK();
+    expand_rows_kernel<<<blocks_for(nnz), kT, 0, st>>>(g->rowptr, n_rows, nnz, rows32.as<int32_t>());
+    GCNB_LAUNCH_CHECK();
+  }
+  return finalize(g, rows32.as<int32_t>(), st);
 }
 
 int from_edges_impl(gcnb_graph** out, int64_t n, int64_t n_edges, const int32_t* src, const int32_t* dst,
@@ -910,6 +1062,8 @@ int from_edges_impl(gcnb_graph** out, int64_t n, int64_t n_edges, const int32_t*
   GCNB_TRY(graph_alloc(g, &g->rowptr, n + 1));
   GCNB_TRY(graph_alloc(g, &g->col, nnz));
   GCNB_TRY(graph_alloc(g, &g->val, nnz));
+  const bool keep_f64 = (flags_in & GCNB_BUILD_KEEP_F64) != 0;
+  if (keep_f64) GCNB_TRY(graph_alloc(g, &g->val64, nnz));
   if (nnz > 0) {
     entries_to_csr_kernel<<<blocks_for(nnz), kT, 0, st>>>(nnz, n, rkey.as<uint64_t>(), rval.as<EntryVal>(),
                                                           rows32.as<int32_t>(), g->col, val64.as<double>());
@@ -917,7 +1071,11 @@ int from_edges_impl(gcnb_graph** out, int64_t n, int64_t n_edges, const int32_t*
   }
   rowptr_from_sorted_kernel<<<blocks_for(n + 1), kT, 0, st>>>(rows32.as<int32_t>(), nnz, n, g->rowptr);
   GCNB_LAUNCH_CHECK();
-  if (n > 0) {
+  if (n > 0 && keep_f64) {
+    if (nnz > 0) GCNB_CUDA(cudaMemcpyAsync(g->val64, val64.p, (size_t)nnz * 8, cudaMemcpyDeviceToDevice, st));
+    normalize_rows_keep_f64_kernel<<<blocks_for(n), kT, 0, st>>>(n, g->rowptr, g->val64, normalize, g->val);
+    GCNB_LAUNCH_CHECK();
+  } else if (n > 0) {
     normalize_rows_kernel<<<blocks_for(n), kT, 0, st>>>(n, g->rowptr, val64.as<double>(), normalize, g->val);
     GCNB_LAUNCH_CHECK();
   }
@@ -953,6 +1111,8 @@ extern "C" void gcnb_graph_free(gcnb_graph* g) {
   cudaFree(g->t_stream_items);
   cudaFree(g->dense_fwd);
   cudaFree(g->dense_bwd);
+  cudaFree(g->val64);
+  cudaFree(g->t_val64);
   if (cur != g->device) cudaSetDevice(cur);
   delete g;
 }
@@ -1007,6 +1167,42 @@ extern "C" int gcnb_graph_from_dense(int64_t n_rows, int64_t n_cols, const float
   GCNB_TRY(check_dims(n_rows, n_cols, 0));
   GCNB_TRY(gcnb_check_device());
   const int s = from_dense_impl(out, n_rows, n_cols, d_a, lda, (cudaStream_t)stream);
+  GCNB_BUILD_EPILOGUE(s);
+}
+
+extern "C" int gcnb_graph_from_coo_f64(int64_t n_rows, int64_t n_cols, int64_t nnz, const int64_t* d_row,
+                                       const int64_t* d_col, const double* d_val, void* stream, gcnb_graph** out) {
+  GCNB_REQUIRE(out != nullptr, "graph_from_coo_f64: out is null");
+  *out = nullptr;
+  GCNB_TRY(check_dims(n_rows, n_cols, nnz));
+  GCNB_REQUIRE((reinterpret_cast<uintptr_t>(d_val) & 7u) == 0, "graph_from_coo_f64: values not 8-byte aligned");
+  GCNB_TRY(gcnb_check_device());
+  *out = new_graph(n_rows, n_cols, nnz);
+  GCNB_REQUIRE(*out != nullptr, "graph: host allocation failed");
+  const int s = from_coo_impl(*out, d_row, d_col, nullptr, (cudaStream_t)stream, true, d_val);
+  GCNB_BUILD_EPILOGUE(s);
+}
+
+extern "C" int gcnb_graph_from_csr_f64(int64_t n_rows, int64_t n_cols, int64_t nnz, const int64_t* d_crow,
+                                       const int64_t* d_col, const double* d_val, void* stream, gcnb_graph** out) {
+  GCNB_REQUIRE(out != nullptr, "graph_from_csr_f64: out is null");
+  *out = nullptr;
+  GCNB_TRY(check_dims(n_rows, n_cols, nnz));
+  GCNB_REQUIRE((reinterpret_cast<uintptr_t>(d_val) & 7u) == 0, "graph_from_csr_f64: values not 8-byte aligned");
+  GCNB_TRY(gcnb_check_device());
+  *out = new_graph(n_rows, n_cols, nnz);
+  GCNB_REQUIRE(*out != nullptr, "graph: host allocation failed");
+  const int s = from_csr_impl(*out, d_crow, d_col, nullptr, (cudaStream_t)stream, true, d_val);
+  GCNB_BUILD_EPILOGUE(s);
+}
+
+extern "C" int gcnb_graph_from_dense_f64(int64_t n_rows, int64_t n_cols, const double* d_a, int64_t lda, void* stream,
+                                         gcnb_graph** out) {
+  GCNB_REQUIRE(out != nullptr, "graph_from_dense_f64: out is null");
+  *out = nullptr;
+  GCNB_TRY(check_dims(n_rows, n_cols, 0));
+  GCNB_TRY(gcnb_check_device());
+  const int s = from_dense_f64_impl(out, n_rows, n_cols, d_a, lda, (cudaStream_t)stream);
   GCNB_BUILD_EPILOGUE(s);
 }
 
@@ -1179,6 +1375,25 @@ extern "C" int gcnb_graph_export_csr(const gcnb_graph* g, int transpose, int32_t
     GCNB_REQUIRE(d_col != nullptr && d_val != nullptr, "graph_export_csr: null output");
     GCNB_CUDA(cudaMemcpyAsync(d_col, v.col, (size_t)v.nnz * 4, cudaMemcpyDeviceToDevice, st));
     GCNB_CUDA(cudaMemcpyAsync(d_val, v.val, (size_t)v.nnz * 4, cudaMemcpyDeviceToDevice, st));
+  }
+  return GCNB_OK;
+}
+
+extern "C" int gcnb_graph_export_csr_f64(const gcnb_graph* g, int transpose, int32_t* d_rowptr, int32_t* d_col,
+                                         double* d_val64, void* stream) {
+  GCNB_REQUIRE(g != nullptr && d_rowptr != nullptr, "graph_export_csr_f64: null argument");
+  if (g->val64 == nullptr) {
+    set_error("graph_export_csr_f64: the handle has no fp64 values (it was built from fp32 data)");
+    return GCNB_E_UNSUPPORTED;
+  }
+  GCNB_REQUIRE(!transpose || g->has_transpose, "graph_export_csr_f64: handle has no transpose");
+  const CsrView& v = transpose ? g->bwd : g->fwd;
+  cudaStream_t st = (cudaStream_t)stream;
+  GCNB_CUDA(cudaMemcpyAsync(d_rowptr, v.rowptr, (size_t)(v.n_rows + 1) * 4, cudaMemcpyDeviceToDevice, st));
+  if (v.nnz > 0) {
+    GCNB_REQUIRE(d_col != nullptr && d_val64 != nullptr, "graph_export_csr_f64: null output");
+    GCNB_CUDA(cudaMemcpyAsync(d_col, v.col, (size_t)v.nnz * 4, cudaMemcpyDeviceToDevice, st));
+    GCNB_CUDA(cudaMemcpyAsync(d_val64, transpose ? g->t_val64 : g->val64, (size_t)v.nnz * 8, cudaMemcpyDeviceToDevice, st));
   }
   return GCNB_OK;
 }

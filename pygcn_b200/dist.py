@@ -1030,6 +1030,9 @@ class DistGraphConvolution(torch.nn.Module):
             self._ops = CudaOps(self.inner.precision)
         if not input.is_cuda:
             raise RuntimeError("DistGraphConvolution runs on CUDA devices only (no CPU fallback)")
+        if input.dtype != torch.float32 or self.inner.weight.dtype != torch.float32:
+            raise RuntimeError("DistGraphConvolution computes in float32 only (got input %s, weight %s); the fp64 layer is "
+                               "the single-GPU GraphConvolution" % (input.dtype, self.inner.weight.dtype))
         ef, eb = self._exchanges(dgraph, input.device)
         assoc = self.association if isinstance(ef, str) else "reference"  # the peer exchange's slots are Fout wide
         return _DistGCNLayerFn.apply(input.contiguous(), self.inner.weight, self.inner.bias, dgraph,

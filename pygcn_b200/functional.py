@@ -5,7 +5,8 @@ Backward : the autograd graph of those lines (SURVEY.md 3.2), hand-written here:
            db = colsum(G); dS = adj^T G; dW = X^T dS; dX = dS W^T  (only what
            ctx.needs_input_grad asks for).
 All arithmetic happens in libgcnb200.so on the current CUDA stream; nothing here falls back
-to PyTorch ops.
+to PyTorch ops.  fp64 operands on an fp64 adjacency (`model.double()`) run the library's fp64 tier
+(the *_f64 entry points): same products, same epilogue, fp64 throughout.
 """
 from __future__ import annotations
 
@@ -26,13 +27,17 @@ def _ld4(f):
     return (f + 3) // 4 * 4
 
 
-def _rowmajor(t):
-    """fp32 2-D tensor with unit column stride (row stride may exceed the width:
+def _ld2(f):
+    return (f + 1) // 2 * 2
+
+
+def _rowmajor(t, dtype=torch.float32):
+    """2-D tensor of `dtype` with unit column stride (row stride may exceed the width:
     the fork passes column-slice views, pygcn/models.py:345)."""
     if t.dim() != 2:
         raise RuntimeError("expected a 2-D tensor, got %d-D" % t.dim())
-    if t.dtype != torch.float32:
-        raise RuntimeError("expected float32, got %s" % t.dtype)
+    if t.dtype != dtype:
+        raise RuntimeError("expected %s, got %s" % (str(dtype).replace("torch.", ""), t.dtype))
     if t.shape[1] > 1 and t.stride(1) != 1:
         t = t.contiguous()
     if t.shape[0] > 1 and t.stride(0) < t.shape[1]:
@@ -84,7 +89,7 @@ def _layer_ws_bytes(lib, graph, fin, fout, precision):
 _ASSOCIATIONS = ("auto", "reference", "aggregate_first")
 
 
-def _aggregate_first(association, graph, xr, fin, fout, need_dx, need_dw):
+def _aggregate_first(association, graph, xr, fin, fout, need_dx, need_dw, lane=4):
     """Which product comes first.  The reference computes adj @ (X @ W) (pygcn/layers.py:33-34); (adj @ X) @ W is the
     same function and the same gradients to fp32 rounding, and its SpMMs gather rows of width fin instead of fout:
     forward one SpMM either way; backward one SpMM of width fout in the reference order (dS = adj^T G, for dW and
@@ -92,10 +97,12 @@ def _aggregate_first(association, graph, xr, fin, fout, need_dx, need_dw):
     "auto" picks the order whose SpMMs move fewer panel columns; ties keep the reference order."""
     if association == "reference" or graph.dense_route:
         return False
-    ok = xr.data_ptr() % 16 == 0 and _ld(xr) % 4 == 0 and _ld(xr) >= _ld4(fin)  # 16-byte gathers of X's rows
+    # 16-byte gathers of X's rows: lane = elements per 16 bytes (4 fp32, 2 fp64)
+    ok = xr.data_ptr() % 16 == 0 and _ld(xr) % lane == 0 and _ld(xr) >= (fin + lane - 1) // lane * lane
     if association == "aggregate_first":
         if not ok:
-            raise RuntimeError("association='aggregate_first' needs 16-byte aligned input rows (stride a multiple of 4)")
+            raise RuntimeError("association='aggregate_first' needs 16-byte aligned input rows (stride a multiple of %d)"
+                               % lane)
         return True
     cost_ref = fout * (2 if (need_dx or need_dw) else 1)
     cost_agg = fin * (2 if need_dx else 1)
@@ -379,6 +386,157 @@ class _GCNLayerBatchedFn(torch.autograd.Function):
         return dx, dw, db, None, None, None
 
 
+class _GCNLayerF64Fn(torch.autograd.Function):
+    """The layer in fp64 (gcnb_layer_forward_f64 / _backward_f64): what `model.double()` computes in the reference, on
+    the handle's fp64 values.  Same association rule as the fp32 layer, with ld2 panels."""
+
+    @staticmethod
+    def forward(ctx, x, weight, bias, graph, relu, mask=None, mask_scale=1.0, association="auto"):
+        lib = _lib.load()
+        dev = x.device
+        f64 = torch.float64
+        fin, fout = weight.shape
+        xr = _rowmajor(x, f64)
+        w = weight.contiguous()
+        b = bias.contiguous() if bias is not None else None
+        agg = _aggregate_first(association, graph, xr, fin, fout, ctx.needs_input_grad[0], ctx.needs_input_grad[1], lane=2)
+        if agg:  # A X, kept for dW = (A X)^T G
+            support = torch.empty((graph.n_rows, _ld2(fin)), dtype=f64, device=dev)
+        else:
+            support = torch.empty((graph.n_cols, _ld2(fout)), dtype=f64, device=dev)
+        out = torch.empty((graph.n_rows, fout), dtype=f64, device=dev)
+        flags = (_lib.LAYER_RELU if relu else 0) | (_lib.LAYER_AGG_FIRST if agg else 0)
+        with _on_device(dev):
+            ws = _ws(lib.gcnb_layer_f64_workspace_bytes(graph._h, fin, fout), dev)
+            _lib.check(lib.gcnb_layer_forward_f64(graph._h, _ptr(xr), _ld(xr), _ptr(w), _ptr(b), fin, fout, flags, _ptr(mask),
+                                                  mask_scale, _ptr(support), _ptr(out), _ptr(ws), ws.numel(),
+                                                  torch.cuda.current_stream(dev).cuda_stream), "gcnb_layer_forward_f64")
+        ctx.graph, ctx.relu, ctx.has_bias, ctx.agg = graph, relu, bias is not None, agg
+        ctx.mask, ctx.mask_scale = mask, mask_scale
+        ctx.save_for_backward(support if agg else xr, w, out if relu else None)
+        return out
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, g):
+        lib = _lib.load()
+        xr, w, y = ctx.saved_tensors
+        graph = ctx.graph
+        dev = g.device
+        f64 = torch.float64
+        fin, fout = w.shape
+        need_dx, need_dw = ctx.needs_input_grad[0], ctx.needs_input_grad[1]
+        need_db = ctx.has_bias and ctx.needs_input_grad[2]
+        gr = _rowmajor(g, f64)
+        flags = (_lib.LAYER_RELU if ctx.relu else 0) | (_lib.LAYER_NEED_DX if need_dx else 0) | (
+            _lib.LAYER_NEED_DW if need_dw else 0) | (_lib.LAYER_NEED_DB if need_db else 0) | (
+            _lib.LAYER_AGG_FIRST if ctx.agg else 0)
+        if ctx.agg:  # scratch for G W^T, only on the way to dX
+            ds = torch.empty((graph.n_rows, _ld2(fin)), dtype=f64, device=dev) if need_dx else None
+        else:
+            ds = torch.empty((graph.n_cols, _ld2(fout)), dtype=f64, device=dev) if (need_dx or need_dw) else None
+        masked = ctx.relu or ctx.mask is not None  # the masked gradient is staged with ld2 rows
+        gm = torch.empty((graph.n_rows, _ld2(fout)), dtype=f64, device=dev) if masked else None
+        dw = torch.empty((fin, fout), dtype=f64, device=dev) if need_dw else None
+        db = torch.empty((fout,), dtype=f64, device=dev) if need_db else None
+        dx = torch.empty((graph.n_cols, fin), dtype=f64, device=dev) if need_dx else None
+        with _on_device(dev):
+            ws = _ws(lib.gcnb_layer_f64_workspace_bytes(graph._h, fin, fout), dev)
+            _lib.check(lib.gcnb_layer_backward_f64(
+                graph._h, _ptr(xr), _ld(xr), _ptr(w), _ptr(gr), _ld(gr), _ptr(y), fin, fout, flags, _ptr(ctx.mask),
+                ctx.mask_scale, _ptr(gm), _ptr(ds), _ptr(dw), _ptr(db), _ptr(dx), fin, _ptr(ws), ws.numel(),
+                torch.cuda.current_stream(dev).cuda_stream), "gcnb_layer_backward_f64")
+        return dx, dw, db, None, None, None, None, None
+
+
+class _GCNLayerBatchedF64Fn(torch.autograd.Function):
+    """_GCNLayerBatchedFn in fp64: one fp64 product over the node-major rows, one fp64 SpMM over the [N, B*Fout] panel."""
+
+    @staticmethod
+    def forward(ctx, x, weight, bias, graph, relu):
+        lib = _lib.load()
+        dev = x.device
+        f64 = torch.float64
+        bsz, n, fin = x.shape
+        fout = weight.shape[1]
+        wide = bsz * fout
+        xn = x.permute(1, 0, 2).contiguous().view(n * bsz, fin)
+        w = weight.contiguous()
+        s2 = torch.empty((n * bsz, fout), dtype=f64, device=dev)
+        out2 = torch.empty((graph.n_rows, wide), dtype=f64, device=dev)
+        brep = bias.detach().repeat(bsz).contiguous() if bias is not None else None
+        with _on_device(dev):
+            sp = _stream_ptr(dev)
+            _gemm_f64(lib, n * bsz, fout, fin, xn, fin, 1, w, fout, 1, s2, fout, dev, sp)
+            _spmm_f64(lib, graph, _lib.SPMM_RELU if relu else 0, s2, wide, wide, brep, out2, wide, dev, sp)
+        ctx.graph, ctx.relu, ctx.has_bias = graph, relu, bias is not None
+        ctx.dims = (bsz, n, fin, fout)
+        ctx.save_for_backward(xn, w, out2 if relu else None)
+        return out2.view(graph.n_rows, bsz, fout).permute(1, 0, 2)
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, g):
+        lib = _lib.load()
+        xn, w, y2 = ctx.saved_tensors
+        graph = ctx.graph
+        bsz, n, fin, fout = ctx.dims
+        wide = bsz * fout
+        dev = g.device
+        f64 = torch.float64
+        need_dx, need_dw, need_db = ctx.needs_input_grad[0], ctx.needs_input_grad[1], ctx.has_bias and ctx.needs_input_grad[2]
+        g2 = g.permute(1, 0, 2).contiguous().view(graph.n_rows, wide)
+        dx = dw = db = None
+        with _on_device(dev):
+            sp = _stream_ptr(dev)
+            gm2 = g2
+            if ctx.relu or need_db:
+                gm2 = torch.empty_like(g2) if ctx.relu else g2
+                dbrep = torch.empty((wide,), dtype=f64, device=dev)
+                _colsum_f64(lib, graph.n_rows, wide, g2, wide, y2 if ctx.relu else None, wide,
+                            gm2 if ctx.relu else None, wide, dbrep, dev, sp)
+                if need_db:  # db = sum over the batch of the per-sample column sums
+                    db = torch.empty((fout,), dtype=f64, device=dev)
+                    _colsum_f64(lib, bsz, fout, dbrep, fout, None, fout, None, fout, db, dev, sp)
+            if need_dw or need_dx:
+                ds2 = torch.empty((graph.n_cols, wide), dtype=f64, device=dev)
+                _spmm_f64(lib, graph, _lib.SPMM_TRANSPOSE, gm2, wide, wide, None, ds2, wide, dev, sp)
+                rows = n * bsz
+                if need_dw:
+                    dw = torch.empty((fin, fout), dtype=f64, device=dev)
+                    _gemm_f64(lib, fin, fout, rows, xn, 1, fin, ds2, fout, 1, dw, fout, dev, sp)
+                if need_dx:
+                    dxn = torch.empty((rows, fin), dtype=f64, device=dev)
+                    _gemm_f64(lib, rows, fin, fout, ds2, fout, 1, w, 1, fout, dxn, fin, dev, sp)
+                    dx = dxn.view(n, bsz, fin).permute(1, 0, 2)
+        return dx, dw, db, None, None
+
+
+def _gemm_f64(lib, m, n, k, a, a_rs, a_cs, b, b_rs, b_cs, out, ldc, dev, sp, bias=None, relu=False):
+    ws = _ws(lib.gcnb_gemm_f64_workspace_bytes(m, n, k), dev)
+    if bias is None and not relu:
+        _lib.check(lib.gcnb_gemm_f64(m, n, k, _ptr(a), a_rs, a_cs, _ptr(b), b_rs, b_cs, _ptr(out), ldc, _ptr(ws), ws.numel(), sp),
+                   "gcnb_gemm_f64")
+    else:
+        _lib.check(lib.gcnb_gemm_f64_ex(m, n, k, _ptr(a), a_rs, a_cs, _ptr(b), b_rs, b_cs, _ptr(out), ldc, _ptr(bias),
+                                        1 if relu else 0, _ptr(ws), ws.numel(), sp), "gcnb_gemm_f64_ex")
+    return out
+
+
+def _spmm_f64(lib, graph, flags, src, ldb, f, bias, out, ldo, dev, sp):
+    ws = _ws(lib.gcnb_spmm_f64_workspace_bytes(graph._h, flags & _lib.SPMM_TRANSPOSE, f), dev)
+    _lib.check(lib.gcnb_spmm_f64(graph._h, flags, _ptr(src), ldb, f, _ptr(bias), None, 0, 1.0, _ptr(out), ldo, _ptr(ws),
+                                 ws.numel(), sp), "gcnb_spmm_f64")
+    return out
+
+
+def _colsum_f64(lib, n_rows, f, g, ldg, y, ldy, gm, ldgm, out, dev, sp):
+    ws = _ws(lib.gcnb_colsum_f64_workspace_bytes(n_rows, f), dev)
+    _lib.check(lib.gcnb_colsum_f64(n_rows, f, _ptr(g), ldg, _ptr(y), ldy, _ptr(gm), ldgm, _ptr(out), _ptr(ws), ws.numel(), sp),
+               "gcnb_colsum_f64")
+    return out
+
+
 def _check_layer_args(x, graph, weight, bias):
     _require_cuda(x, "input")
     _require_cuda(weight, "weight")
@@ -392,14 +550,17 @@ def _check_layer_args(x, graph, weight, bias):
         raise RuntimeError(
             "size mismatch: adj is %dx%d but input has %d rows" % (graph.n_rows, graph.n_cols, x.shape[0])
         )
-    if x.dtype != torch.float32 or weight.dtype != torch.float32:
-        raise RuntimeError("expected float32 input and weight (the reference layer is fp32)")
+    if x.dtype not in (torch.float32, torch.float64):
+        raise RuntimeError("expected float32 or float64 input, got %s" % x.dtype)
+    if weight.dtype != x.dtype or graph.dtype != x.dtype or (bias is not None and bias.dtype != x.dtype):
+        raise RuntimeError("input (%s), weight (%s), bias (%s) and adj (%s) must have one dtype" % (
+            x.dtype, weight.dtype, None if bias is None else bias.dtype, graph.dtype))
     if x.device != graph.device or weight.device != graph.device:
         raise RuntimeError("input (%s), weight (%s) and adj (%s) must be on the same device" %
                            (x.device, weight.device, graph.device))
     if bias is not None:
-        if bias.shape != (weight.shape[1],) or bias.dtype != torch.float32 or bias.device != graph.device:
-            raise RuntimeError("bias must be a float32 [%d] tensor on %s" % (weight.shape[1], graph.device))
+        if bias.shape != (weight.shape[1],) or bias.device != graph.device:
+            raise RuntimeError("bias must be a %s [%d] tensor on %s" % (x.dtype, weight.shape[1], graph.device))
 
 
 def gcn_layer(input, adj, weight, bias=None, relu=False, precision="auto", dropout_mask=None, dropout_p=0.0,
@@ -416,16 +577,23 @@ def gcn_layer(input, adj, weight, bias=None, relu=False, precision="auto", dropo
     association: "auto" (default) computes (adj @ input) @ weight instead of the reference's adj @ (input @ weight)
     when that moves fewer bytes through the SpMMs (in_features < out_features; see _aggregate_first) -- same result
     to fp32 rounding; "reference" / "aggregate_first" force one order.
+    fp64 input, weight, bias and adj (all one dtype, as torch requires) compute the layer in fp64; precision must then be
+    "auto".
     """
     if association not in _ASSOCIATIONS:
         raise ValueError("association must be one of %s, got %r" % (_ASSOCIATIONS, association))
     graph = as_graph(adj)
+    f64 = isinstance(input, torch.Tensor) and input.dtype == torch.float64
+    if f64 and precision != "auto":
+        raise ValueError("precision=%r selects an fp32 kernel tier; with float64 operands precision must be 'auto'" % (precision,))
     if input.dim() == 3:  # [B, N, Fin]: the batch shares the adjacency (pygcn/models.py:343-349)
         if dropout_mask is not None:
             raise NotImplementedError("the fused dropout mask is not available for batched input")
         if input.shape[0] == 0:
             return input.new_empty((0, graph.n_rows, weight.shape[1]))
         _check_layer_args(input[0], graph, weight, bias)
+        if f64:
+            return _GCNLayerBatchedF64Fn.apply(input, weight, bias, graph, bool(relu))
         return _GCNLayerBatchedFn.apply(input, weight, bias, graph, bool(relu), _PRECISIONS[precision])
     _check_layer_args(input, graph, weight, bias)
     if precision == "bf16" and not graph.dense_route:
@@ -440,6 +608,8 @@ def gcn_layer(input, adj, weight, bias=None, relu=False, precision="auto", dropo
             raise RuntimeError("dropout_mask must be a [%d, %d] tensor on %s" % (graph.n_rows, weight.shape[1], graph.device))
         mask = dropout_mask.to(torch.uint8).contiguous()
         scale = 1.0 / (1.0 - dropout_p)
+    if f64:
+        return _GCNLayerF64Fn.apply(input, weight, bias, graph, bool(relu), mask, scale, association)
     return _GCNLayerFn.apply(input, weight, bias, graph, bool(relu), _PRECISIONS[precision], mask, scale, association)
 
 
@@ -481,6 +651,35 @@ class _SpmmFn(torch.autograd.Function):
         return out, None
 
 
+class _SpmmF64Fn(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, dense, graph):
+        lib = _lib.load()
+        dev = dense.device
+        d = _rowmajor(dense, torch.float64)
+        f = d.shape[1]
+        out = torch.empty((graph.n_rows, f), dtype=torch.float64, device=dev)
+        ctx.graph = graph
+        if f > 0 and graph.n_rows > 0:
+            with torch.cuda.device(dev):
+                _spmm_f64(lib, graph, 0, d, _ld(d), f, None, out, f, dev, _stream_ptr(dev))
+        return out
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, g):
+        lib = _lib.load()
+        graph = ctx.graph
+        dev = g.device
+        gr = _rowmajor(g, torch.float64)
+        f = gr.shape[1]
+        out = torch.empty((graph.n_cols, f), dtype=torch.float64, device=dev)
+        if f > 0 and graph.n_cols > 0:
+            with torch.cuda.device(dev):
+                _spmm_f64(lib, graph, _lib.SPMM_TRANSPOSE, gr, _ld(gr), f, None, out, f, dev, _stream_ptr(dev))
+        return out, None
+
+
 def spmm(adj, dense):
     """Drop-in for `torch.spmm(adj, dense)` as the layer uses it (pygcn/layers.py:34).
 
@@ -493,10 +692,14 @@ def spmm(adj, dense):
     if dense.dim() != 2 or dense.shape[0] != graph.n_cols:
         raise RuntimeError("mat1 and mat2 shapes cannot be multiplied (%dx%d and %s)" %
                            (graph.n_rows, graph.n_cols, "x".join(str(s) for s in dense.shape)))
-    if dense.dtype != torch.float32:
-        raise RuntimeError("expected float32 dense operand, got %s" % dense.dtype)
+    if dense.dtype not in (torch.float32, torch.float64):
+        raise RuntimeError("expected float32 or float64 dense operand, got %s" % dense.dtype)
+    if dense.dtype != graph.dtype:
+        raise RuntimeError("adj (%s) and dense (%s) must have one dtype" % (graph.dtype, dense.dtype))
     if dense.device != graph.device:
         raise RuntimeError("adj (%s) and dense (%s) must be on the same device" % (graph.device, dense.device))
+    if dense.dtype == torch.float64:
+        return _SpmmF64Fn.apply(dense, graph)
     return _SpmmFn.apply(dense, graph)
 
 
@@ -528,7 +731,8 @@ def load_adj(avg_visits, precision="auto"):
 
 
 def mm(a, b, precision="auto"):
-    """`torch.mm(a, b)` through gcnb_gemm (no autograd); used by tests and the benchmark."""
+    """`torch.mm(a, b)` through gcnb_gemm (no autograd); used by tests and the benchmark.  fp64 a and b run the fp64
+    product (gcnb_gemm_f64, precision "auto" only)."""
     lib = _lib.load()
     _require_cuda(a, "a")
     _require_cuda(b, "b")
@@ -536,6 +740,16 @@ def mm(a, b, precision="auto"):
         raise RuntimeError("mat1 and mat2 shapes cannot be multiplied")
     m, k = a.shape
     n = b.shape[1]
+    if a.dtype == torch.float64 or b.dtype == torch.float64:
+        if a.dtype != b.dtype:
+            raise RuntimeError("expected both operands of one dtype, got %s and %s" % (a.dtype, b.dtype))
+        if precision != "auto":
+            raise ValueError("with float64 operands precision must be 'auto', got %r" % (precision,))
+        out = torch.empty((m, n), dtype=torch.float64, device=a.device)
+        with torch.cuda.device(a.device):
+            _gemm_f64(lib, m, n, k, a, a.stride(0), a.stride(1), b, b.stride(0), b.stride(1), out, max(n, 1), a.device,
+                      _stream_ptr(a.device))
+        return out
     out = torch.empty((m, n), dtype=torch.float32, device=a.device)
     prec = _PRECISIONS[precision]
     with torch.cuda.device(a.device):

@@ -35,10 +35,12 @@ def _require_cuda(t, what):
 class Graph:
     """Opaque handle to a gcnb_graph living in HBM.  Accepted wherever `adj` is."""
 
-    def __init__(self, handle, device, source="unknown"):
+    def __init__(self, handle, device, source="unknown", dtype=torch.float32):
         self._h = ctypes.c_void_p(handle)
         self.device = torch.device(device)
         self.source = source
+        # torch.float64: the handle keeps fp64 values (and their fp32 rounding); layers on it compute in fp64
+        self.dtype = dtype
         info = _lib.GraphInfo()
         _lib.check(_lib.load().gcnb_graph_get_info(self._h, ctypes.byref(info)), "gcnb_graph_get_info")
         self.n_rows, self.n_cols, self.nnz = int(info.n_rows), int(info.n_cols), int(info.nnz)
@@ -53,12 +55,15 @@ class Graph:
 
     # ------------------------------------------------------------------ constructors
     @classmethod
-    def from_edges(cls, src, dst, num_nodes, symmetrize=True, self_loops=True, row_normalize=True):
+    def from_edges(cls, src, dst, num_nodes, symmetrize=True, self_loops=True, row_normalize=True, dtype=torch.float32):
         """Edge list -> (optionally) max-symmetrised, + I, row-normalised adjacency.
 
         With all three flags set this is the reference's Cora pipeline
-        (pygcn/utils.py:360-368, 390-397, 407-414) bit for bit.
+        (pygcn/utils.py:360-368, 390-397, 407-414) bit for bit.  dtype=torch.float64 keeps the fp64 values
+        `normalize` computes before the cast of utils.py:409 (an fp64 handle).
         """
+        if dtype not in (torch.float32, torch.float64):
+            raise ValueError("dtype must be torch.float32 or torch.float64, got %s" % (dtype,))
         _require_cuda(src, "src")
         _require_cuda(dst, "dst")
         if src.dim() != 1 or src.shape != dst.shape:
@@ -66,8 +71,7 @@ class Graph:
         src = src.to(torch.int32).contiguous()
         dst = dst.to(torch.int32).contiguous()
         flags = (_lib.BUILD_SYMMETRIZE if symmetrize else 0) | (_lib.BUILD_SELF_LOOPS if self_loops else 0) | (
-            _lib.BUILD_ROW_NORMALIZE if row_normalize else 0
-        )
+            _lib.BUILD_ROW_NORMALIZE if row_normalize else 0) | (_lib.BUILD_KEEP_F64 if dtype == torch.float64 else 0)
         out = ctypes.c_void_p()
         with torch.cuda.device(src.device):
             st = _lib.load().gcnb_graph_from_edges(
@@ -75,16 +79,18 @@ class Graph:
                 ctypes.byref(out),
             )
         _lib.check(st, "gcnb_graph_from_edges")
-        return cls(out.value, src.device, "edges")
+        return cls(out.value, src.device, "edges", dtype)
 
     @classmethod
     def from_torch(cls, adj):
-        """torch adjacency (sparse COO, sparse CSR or dense strided, fp32) -> Graph."""
+        """torch adjacency (sparse COO, sparse CSR or dense strided; fp32, or fp64 for an fp64 handle) -> Graph."""
         _require_cuda(adj, "adj")
         if adj.dim() != 2:
             raise RuntimeError("adj must be a matrix, got %d-D" % adj.dim())
-        if adj.dtype != torch.float32:
-            raise RuntimeError("adj must be float32 (the reference builds FloatTensors), got %s" % adj.dtype)
+        if adj.dtype not in (torch.float32, torch.float64):
+            raise RuntimeError("adj must be float32 (the reference builds FloatTensors) or float64, got %s" % adj.dtype)
+        f64 = adj.dtype == torch.float64
+        sfx = "_f64" if f64 else ""
         lib = _lib.load()
         out = ctypes.c_void_p()
         n_rows, n_cols = adj.shape
@@ -97,15 +103,15 @@ class Graph:
                 val = adj._values().contiguous()
                 row = idx[0].contiguous()
                 col = idx[1].contiguous()
-                st = lib.gcnb_graph_from_coo(n_rows, n_cols, val.numel(), row.data_ptr(), col.data_ptr(),
-                                             val.data_ptr(), sp, ctypes.byref(out))
+                st = getattr(lib, "gcnb_graph_from_coo" + sfx)(n_rows, n_cols, val.numel(), row.data_ptr(), col.data_ptr(),
+                                                               val.data_ptr(), sp, ctypes.byref(out))
                 src = "coo"
             elif adj.layout == torch.sparse_csr:
                 crow = adj.crow_indices().to(torch.int64).contiguous()
                 col = adj.col_indices().to(torch.int64).contiguous()
                 val = adj.values().contiguous()
-                st = lib.gcnb_graph_from_csr(n_rows, n_cols, val.numel(), crow.data_ptr(), col.data_ptr(),
-                                             val.data_ptr(), sp, ctypes.byref(out))
+                st = getattr(lib, "gcnb_graph_from_csr" + sfx)(n_rows, n_cols, val.numel(), crow.data_ptr(), col.data_ptr(),
+                                                               val.data_ptr(), sp, ctypes.byref(out))
                 src = "csr"
             elif adj.layout == torch.strided:
                 a = adj if adj.stride(1) == 1 or n_cols <= 1 else adj.contiguous()
@@ -113,17 +119,17 @@ class Graph:
                 if lda < n_cols:
                     a = a.contiguous()
                     lda = n_cols
-                st = lib.gcnb_graph_from_dense(n_rows, n_cols, a.data_ptr(), lda, sp, ctypes.byref(out))
+                st = getattr(lib, "gcnb_graph_from_dense" + sfx)(n_rows, n_cols, a.data_ptr(), lda, sp, ctypes.byref(out))
                 src = "dense"
             else:
                 raise RuntimeError("unsupported adjacency layout %s" % adj.layout)
-        _lib.check(st, "gcnb_graph_from_" + src)
-        return cls(out.value, adj.device, src)
+        _lib.check(st, "gcnb_graph_from_" + src + sfx)
+        return cls(out.value, adj.device, src, adj.dtype)
 
     # ------------------------------------------------------------------ exports
     def to_sparse_coo(self):
         """torch sparse COO tensor in the exact layout utils.py:407-414 returns
-        (int64 [2,nnz] indices, row-major / columns ascending, fp32 values, uncoalesced flag)."""
+        (int64 [2,nnz] indices, row-major / columns ascending, fp32 values -- fp64 on an fp64 handle -- uncoalesced flag)."""
         idx = torch.empty((2, self.nnz), dtype=torch.int64, device=self.device)
         val = torch.empty((self.nnz,), dtype=torch.float32, device=self.device)
         with torch.cuda.device(self.device):
@@ -131,19 +137,24 @@ class Graph:
                 _lib.load().gcnb_graph_export_coo(self._h, idx.data_ptr(), val.data_ptr(), _stream_ptr(self.device)),
                 "gcnb_graph_export_coo",
             )
+        if self.dtype == torch.float64:  # the COO values are the CSR's, in the same order
+            val = self.csr()[2]
         return torch.sparse_coo_tensor(idx, val, (self.n_rows, self.n_cols), check_invariants=False)
 
     def csr(self, transpose=False):
-        """(rowptr int32, col int32, val fp32) copies of the device CSR (or of the CSR of A^T)."""
+        """(rowptr int32, col int32, val) copies of the device CSR (or of the CSR of A^T); val is fp32, or fp64 on an
+        fp64 handle."""
         rows = self.n_cols if transpose else self.n_rows
+        f64 = self.dtype == torch.float64
         rowptr = torch.empty((rows + 1,), dtype=torch.int32, device=self.device)
         col = torch.empty((self.nnz,), dtype=torch.int32, device=self.device)
-        val = torch.empty((self.nnz,), dtype=torch.float32, device=self.device)
+        val = torch.empty((self.nnz,), dtype=self.dtype, device=self.device)
+        name = "gcnb_graph_export_csr_f64" if f64 else "gcnb_graph_export_csr"
         with torch.cuda.device(self.device):
             _lib.check(
-                _lib.load().gcnb_graph_export_csr(self._h, 1 if transpose else 0, rowptr.data_ptr(), col.data_ptr(),
-                                                  val.data_ptr(), _stream_ptr(self.device)),
-                "gcnb_graph_export_csr",
+                getattr(_lib.load(), name)(self._h, 1 if transpose else 0, rowptr.data_ptr(), col.data_ptr(),
+                                           val.data_ptr(), _stream_ptr(self.device)),
+                name,
             )
         return rowptr, col, val
 
@@ -152,9 +163,10 @@ class Graph:
         return (self.n_rows, self.n_cols)
 
     def __repr__(self):
-        return "Graph(%d x %d, nnz=%d, bins=%s, long_chunks=%d, sym_pattern=%s, %s%s, %.1f MB)" % (
+        return "Graph(%d x %d, nnz=%d, bins=%s, long_chunks=%d, sym_pattern=%s, %s%s%s, %.1f MB)" % (
             self.n_rows, self.n_cols, self.nnz, self.bin_rows, self.n_long_chunks, self.pattern_symmetric,
-            "dense route, " if self.dense_route else "", self.device, self.device_bytes / 1e6,
+            "dense route, " if self.dense_route else "", "fp64, " if self.dtype == torch.float64 else "", self.device,
+            self.device_bytes / 1e6,
         )
 
 
